@@ -34,6 +34,9 @@ Secondary lines (not the driver's metric; `profiles/` holds one of each):
   --workload gmf       NCF-GMF training step (daisy_gmf_step) on the ml-100k shape, batch 256
   --workload bprfm     BPR-FM training step (daisy_bprfm_adagrad_step) on the ml-100k shape, batch 4 096
   --phases / --trace   per-phase device times (serialised) / timeline of bookkeeping vs table kernels
+  --dump-outputs DIR   config3 / config4: after the timed steps, the loss of the last timed call and a fixed sample of
+                     the trained tables as DIR/<name>.npy (sample_outputs), so that two builds can be compared on the same
+                     seeded inputs
 """
 from __future__ import annotations
 
@@ -46,6 +49,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                  # the benchmark writes nothing into the tree it runs from
 
 import numpy as np  # noqa: E402
 
@@ -67,6 +71,36 @@ UNIT = "triples/s"
 def alg_bytes_per_triple(dim):
     """SURVEY.md 8d: gather 3 rows + scatter 3 rows (fp32) + 12 B of ids."""
     return 24 * dim + 12
+
+
+DUMP_ROWS = 16_384
+
+
+def sample_outputs(model, last_batch, loss, seed=2019):
+    """What a caller of the timed step holds after its last call, as a fixed sample small enough to store (about 42 MB
+    at D = 128): the loss the call returned, the rows of the last batch's first DUMP_ROWS triples (rows that step
+    updated; hot items included) and DUMP_ROWS rows of each table at ids drawn with a fixed seed.  The tables must be
+    materialized."""
+    import torch
+    P, Q = model.embed_user.weight.detach(), model.embed_item.weight.detach()
+    rng = np.random.default_rng(seed)
+    uid = torch.from_numpy(np.sort(rng.choice(P.shape[0], min(DUMP_ROWS, P.shape[0]), replace=False)))
+    iid = torch.from_numpy(np.sort(rng.choice(Q.shape[0], min(DUMP_ROWS, Q.shape[0]), replace=False)))
+    tri = last_batch[:DUMP_ROWS].long()
+
+    def rows(table, ids):
+        return table.index_select(0, ids.to(table.device)).cpu().numpy().astype(np.float32)
+
+    return {"loss": loss.detach().reshape(1).cpu().numpy().astype(np.float64),
+            "user_rows": rows(P, uid), "item_rows": rows(Q, iid),
+            "last_batch_user_rows": rows(P, tri[:, 0]), "last_batch_pos_item_rows": rows(Q, tri[:, 1]),
+            "last_batch_neg_item_rows": rows(Q, tri[:, 2])}
+
+
+def write_outputs(dirname, outputs):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -280,6 +314,9 @@ def run_single(args):
     h.set_timing(0)
     model.check()
     value = B * K / (ms_total * 1e-3)
+    outputs = None
+    if args.dump_outputs:                       # the e2e pass below trains on: sample the timed pass's result now
+        outputs = sample_outputs(model, devtri[W + K - 1], loss_dev[W if args.epoch_api else W + K - 1])
 
     # ---- e2e: host triples through the public API, loss read back every step ----
     def e2e_pass(first, count):
@@ -379,6 +416,8 @@ def run_single(args):
         line["phase_ms"] = {k: round(v, 4) for k, v in phases.items()}
     if trace:
         line["trace_ms(book_begin,book_end,kernels_begin,kernels_end)"] = trace
+    if outputs:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -1072,11 +1111,17 @@ def main():
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N > 1: peer = fused peer-memory step (product), nccl = all-to-all exchange (comparison)")
     ap.add_argument("--cpu-budget", type=float, default=25.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="config3/config4: after the timed steps, write the loss of the last timed call and a fixed "
+                         "sample of the trained table rows as DIR/<name>.npy (float32 / float64, about 42 MB)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "b200" or args.gpus > 1 or world > 1
+                              or args.workload not in ("config3", "config4")):
+        ap.error("--dump-outputs: single-GPU config3 / config4 only")
     if args.impl == "reference":
         return run_reference(args)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus > 1 or world > 1:
         from bench_sharded import bench_sharded
         return bench_sharded(args, CFG5, METRIC, UNIT)

@@ -12,7 +12,8 @@ ml100k_split.npz     train / test pairs of config 1: leave-one-out by latest tim
                      the numpy restatement in recommend_lib_b200/data.py is asserted equal.
 bpr_small.npz        3 steps of the reference BPR + optim.SGD on a tiny table with heavy in-batch
                      duplicates (BPRMFRecommender.py:28-50,154,172-176).
-bpr_config1_step.npz first step of config 1 (943 x 1682, D 64, B 4096, lr .01, wd .001).
+bpr_config1_step.npz first step of config 1 (943 x 1682, D 64, B 4096, lr .01, wd .001): tables
+                     before the step, the batch and the loss; bpr_config1_step_after.npz: the tables after it.
 bpr_eval_small.npz   reference metric_eval (util/metrics.py:46-66,88-94) on a tiny model.
 bpr_ml100k_traj.json 20-epoch config-1 trajectory of the reference loop fed by the
                      deterministic sampler: epoch loss, HR@10, NDCG@10.
@@ -158,8 +159,9 @@ def make_config1_step(train_pairs, user_num, item_num):
     batch = next(iter(sampler.batches(0, 4096)))
     losses = ref_steps(model, [batch], 0.01, 0.001)
     P1, Q1 = tables(model)
-    np.savez_compressed(f"{HERE}/bpr_config1_step.npz", P0=P0, Q0=Q0, P1=P1, Q1=Q1, loss=losses[0],
-                        batch=batch, batch_sha=sha(batch))
+    # two files keep each fixture under 1 MB (the tables before and after the step are 1.3 MB together)
+    np.savez_compressed(f"{HERE}/bpr_config1_step.npz", P0=P0, Q0=Q0, loss=losses[0], batch=batch, batch_sha=sha(batch))
+    np.savez_compressed(f"{HERE}/bpr_config1_step_after.npz", P1=P1, Q1=Q1)
     print("config1 step loss", losses[0], "batch sha", sha(batch))
 
 

@@ -1,10 +1,7 @@
-"""GPU parity tests of the funk-SVD / RSVD path against the reference's compiled Cython extension (golden fixtures,
-and oracle/_ref live when it travelled) and the C oracle.  float64 on both sides; the device computes the dot
-product with a warp tree instead of a left-to-right loop, so agreement is to rounding (1e-9 relative stated here),
-not bit-exact; the sequential update ORDER is the reference's."""
-import contextlib
-import io
-
+"""GPU parity tests of the funk-SVD / RSVD path against the reference's compiled Cython extension (golden fixtures)
+and the C oracle.  float64 on both sides; the device computes the dot product with a warp tree instead of a
+left-to-right loop, so agreement is to rounding (1e-9 relative stated here), not bit-exact; the sequential update ORDER
+is the reference's."""
 import numpy as np
 import pytest
 
@@ -183,26 +180,6 @@ def test_batched_groups_match_the_link_by_link_schedule_and_are_reproducible(mon
         o = ofit(p0, q0)
         for x, k in zip(runs["b1"], names):
             assert rel_err(x, o[k]) <= TOL, k
-
-
-def test_live_reference_extension_when_present():
-    from oracle.build_ref import load_ref
-    from recommend_lib_b200.mf import RSVD
-    m = load_ref()
-    if m is None:
-        pytest.skip("oracle/_ref not available on this box")
-    rng = np.random.default_rng(4)
-    U, I, D, N = 80, 60, 24, 3000
-    df = pd.DataFrame({"user": rng.integers(0, U, N), "item": rng.integers(0, I, N),
-                       "rating": rng.integers(1, 6, N).astype(float)})
-    np.random.seed(3)
-    r = m.RSVD(U, I, n_factors=D, n_epochs=2, version=2, verbose=True)
-    with contextlib.redirect_stdout(io.StringIO()):
-        r.fit(df)
-    np.random.seed(3)
-    a = RSVD(U, I, n_factors=D, n_epochs=2, version=2, verbose=False)
-    a.fit(df)
-    assert rel_err(a.ui, r.ui) <= TOL and rel_err(a.vj, r.vj) <= TOL and rel_err(a.ci, r.ci) <= TOL
 
 
 def test_many_items_per_warp_and_wide_rows():

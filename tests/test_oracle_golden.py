@@ -87,7 +87,7 @@ def test_forward_matches_reference(golden):
 
 
 def test_config1_first_step(golden):
-    g = golden("bpr_config1_step.npz")
+    g = {**golden("bpr_config1_step.npz"), **golden("bpr_config1_step_after.npz")}
     P1, Q1, loss = bpr_oracle.bpr_step_closed_form(g["P0"], g["Q0"], g["batch"], 0.01, 0.001, np.float64)
     assert rel_err(P1, g["P1"]) < 1e-6 and rel_err(Q1, g["Q1"]) < 1e-6
     assert abs(loss - float(g["loss"])) / float(g["loss"]) < 1e-6
@@ -170,24 +170,15 @@ def test_predict_rejects_invalid_codes(golden):
         mf_oracle.predict(0, int(g["I"]), g["svd_b_pu"], g["svd_b_qi"], g["svd_b_bu"], g["svd_b_bi"], True)
 
 
-def test_live_reference_extension_when_present():
-    """When oracle/_ref is built (build container, or shipped to the GPU box) re-check on fresh data."""
-    from oracle.build_ref import load_ref
-    m = load_ref()
-    if m is None:
-        pytest.skip("oracle/_ref not available")
-    import pandas as pd
-    rng = np.random.default_rng(5)
-    U, I, D, N = 30, 20, 6, 300
-    users, items = rng.integers(0, U, N), rng.integers(0, I, N)
-    ratings = rng.integers(1, 6, N).astype(float)
-    np.random.seed(1)
-    a = m.SVD(U, I, n_factors=D, n_epochs=2, verbose=False)
-    a.fit(pd.DataFrame({"user": users, "item": items, "rating": ratings}))
-    np.random.seed(1)
-    pu0, qi0 = mf_oracle.draw_init(U, I, D)
-    o = mf_oracle.svd_fit(users, items, ratings, pu0, qi0, n_epochs=2)
-    assert np.array_equal(o["pu"], a.pu) and np.array_equal(o["qi"], a.qi)
+def test_seeded_draw_and_fit_match_the_reference_extension_golden(golden):
+    """The reference's SVD.fit draws its start from the global numpy RNG: draw_init under the seed of the fixture's run,
+    then svd_fit, ends bit for bit where the compiled reference ended (mf_small.npz, seed 2019)."""
+    g = golden("mf_small.npz")
+    np.random.seed(2019)
+    pu0, qi0 = mf_oracle.draw_init(int(g["U"]), int(g["I"]), int(g["D"]))
+    assert np.array_equal(pu0, g["svd_b_pu0"]) and np.array_equal(qi0, g["svd_b_qi0"])
+    o = mf_oracle.svd_fit(g["users"], g["items"], g["ratings"], pu0, qi0, n_epochs=int(g["E"]))
+    assert np.array_equal(o["pu"], g["svd_b_pu"]) and np.array_equal(o["qi"], g["svd_b_qi"])
 
 
 # ------------------------------------------------------------------------------------------------
