@@ -91,7 +91,11 @@ DAISY_API int daisy_bpr_step(daisy_handle_t h, float *P, float *Q, const int32_t
  * daisy_bpr_step assumes `triples` may still be being produced by earlier work on `stream` and orders its
  * bookkeeping after that work (which also orders it after step n: no overlap).  Declare with on = 1 that device
  * triples passed to daisy_bpr_step are complete at call time (e.g. batches uploaded and synchronised up front)
- * to get the overlap.  daisy_bpr_step_host always overlaps (host memory is complete at call time). */
+ * to get the overlap.  daisy_bpr_step_host always overlaps (host memory is complete at call time).
+ * The flag stays set until it is changed.  It is read by daisy_bpr_step, daisy_gmf_step and the row-sharded steps
+ * (daisy_bpr_shard_step, daisy_shard_step, daisy_shard_compute, daisy_shard_prepare) only.  daisy_bpr_epoch and
+ * daisy_gmf_epoch with device input order their bookkeeping once per call behind the work already on `stream`, and
+ * daisy_bpr_adam_step and daisy_bprfm_adagrad_step at every call, whatever the flag says. */
 DAISY_API int daisy_set_inputs_ready(daisy_handle_t h, int on);
 
 /* Same step fed from HOST memory (the reference's `user.cuda(); item_i.cuda(); item_j.cuda()`,

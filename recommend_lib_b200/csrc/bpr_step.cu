@@ -160,9 +160,10 @@ extern "C" int daisy_bpr_epoch(daisy_handle_t h, float *P, float *Q, const int32
     DAISY_REQUIRE(n >= 0 && batch > 0, DAISY_EINVAL, "epoch of %lld triples in batches of %lld", (long long)n, (long long)batch);
     int rc = check_step_args(h, P, Q, triples, batch < n ? batch : n);
     if (rc) return rc;
-    if (!on_host && n > 0 && h->pipeline && !h->inputs_ready) {
+    if (!on_host && n > 0 && h->pipeline) {
         // the triples are complete once the work already queued on `stream` is: order the bookkeeping stream behind
-        // it ONCE, then every step's bookkeeping may run ahead of the previous step's kernels
+        // it ONCE, then every step's bookkeeping may run ahead of the previous step's kernels.  Whatever the handle's
+        // inputs-ready flag says: it describes the triples of daisy_bpr_step calls, not these.
         DeviceGuard g(h->device);
         DAISY_CUDA(cudaEventRecord(h->ev_call, (cudaStream_t)stream));
         DAISY_CUDA(cudaStreamWaitEvent(h->side_stream, h->ev_call, 0));
@@ -201,8 +202,8 @@ extern "C" int daisy_bpr_adam_step(daisy_handle_t h, float *P, float *Q, float *
     opt.step_size = (float)((double)lr * sqrt(bc2) / bc1);
     opt.eps = eps;
     opt.D4 = h->D / 4;
-    return run_step<AdamOpt>(h, P, Q, triples, B, opt, 1.0f, loss_accum, (cudaStream_t)stream, nullptr,
-                             h->inputs_ready != 0);
+    // the triples may have been produced by earlier work on `stream` (the inputs-ready flag is daisy_bpr_step's)
+    return run_step<AdamOpt>(h, P, Q, triples, B, opt, 1.0f, loss_accum, (cudaStream_t)stream, nullptr, false);
 }
 
 extern "C" int daisy_bprfm_adagrad_step(daisy_handle_t h, float *E, float *acc, const int32_t *triples, int64_t B, float lr,
@@ -223,6 +224,6 @@ extern "C" int daisy_bprfm_adagrad_step(daisy_handle_t h, float *E, float *acc, 
     opt.eps = eps;
     opt.D4 = h->D / 4;
     opt.const_e = h->D / 4 - 1;                             // the last float4 of a row: [x, 0, 0, 0]
-    return run_step<AdagradOpt>(h, P, Q, triples, B, opt, 1.0f, loss_accum, (cudaStream_t)stream, nullptr,
-                                h->inputs_ready != 0);
+    // the triples may have been produced by earlier work on `stream` (the inputs-ready flag is daisy_bpr_step's)
+    return run_step<AdagradOpt>(h, P, Q, triples, B, opt, 1.0f, loss_accum, (cudaStream_t)stream, nullptr, false);
 }

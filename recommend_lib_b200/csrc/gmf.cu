@@ -272,7 +272,7 @@ extern "C" int daisy_gmf_epoch(daisy_handle_t h, float *P, float *Q, float *w, f
     DeviceGuard g(h->device);
     DAISY_REQUIRE(g.ok, DAISY_ECUDA, "cannot select device %d", h->device);
     cudaStream_t s = (cudaStream_t)stream;
-    if (!on_host && n > 0 && h->pipeline && !h->inputs_ready) {  // cf. daisy_bpr_epoch
+    if (!on_host && n > 0 && h->pipeline) {  // cf. daisy_bpr_epoch: whatever the inputs-ready flag says
         DAISY_CUDA(cudaEventRecord(h->ev_call, s));
         DAISY_CUDA(cudaStreamWaitEvent(h->side_stream, h->ev_call, 0));
     }
