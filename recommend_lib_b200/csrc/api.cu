@@ -5,6 +5,7 @@
 #include <cub/device/device_scan.cuh>
 
 #include "ctx.cuh"
+#include "ref_sort.cuh"
 
 static thread_local char g_err[512] = "";
 
@@ -130,6 +131,7 @@ extern "C" int daisy_create(daisy_handle_t *out, int device, int64_t user_num, i
             A(book[i].ukey_s, B); A(book[i].qkey_s, 2 * B);
             A(book[i].uslot, B); A(book[i].jslot, B); A(book[i].islot, B);
             A(book[i].longs, 2 + 5 * (size_t)h->longs_cap);
+            A(book[i].counts, 2);
         }
         A(key_in, 3 * B); A(val_in, 3 * B); A(val_out, 3 * B); A(key_out, 3 * B);
         A(ukey_in, B); A(uval_in, B); A(uval_out, B);
@@ -140,6 +142,10 @@ extern "C" int daisy_create(daisy_handle_t *out, int device, int64_t user_num, i
         A(loss_part, B);
         A(ticket, (size_t)h->longs_cap);
         A(mid_buf, 4 * 3 * (size_t)h->mid_cap);
+        if (h->merged_sort != 0) {  // item refs name at most max(I, 2B) rows: the sharded step's cache rows stand in for I
+            h->ref_rows = user_num + (item_num > 2 * max_batch ? item_num : 2 * max_batch);
+            A(ref_ws, sizeof(DsortState) / 4 + 2 * (size_t)((h->ref_rows + 31) / 32) + dsort_status_words(3 * max_batch));
+        }
     }
 #undef A
     if (!rc && B > 0) {
@@ -208,12 +214,12 @@ extern "C" int daisy_destroy(daisy_handle_t h) {
     void *ptrs[] = {h->triples, h->key_in, h->val_in, h->val_out, h->ukey_in, h->uval_in, h->uval_out, h->ikey_in,
                     h->ikey_out, h->ival_in, h->ival_out, h->stageU, h->stageQ, h->stage2, h->loss_part, h->key_out,
                     h->err, h->cub_tmp, h->ticket, h->mid_buf, h->gradP, h->gradQ, h->wpart, h->scores, h->sel_hist, h->own_key, h->own_key_s, h->own_val, h->own_val_s,
-                    h->own_tmp};
+                    h->own_tmp, h->ref_ws};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (int i = 0; i < DAISY_NSETS; ++i) {
         void *bp[] = {h->book[i].st, h->book[i].ukey_s, h->book[i].qkey_s, h->book[i].uslot, h->book[i].jslot,
-                      h->book[i].islot, h->book[i].longs};
+                      h->book[i].islot, h->book[i].longs, h->book[i].counts};
         for (void *p : bp)
             if (p) cudaFree(p);
         if (h->book[i].ready) cudaEventDestroy(h->book[i].ready);

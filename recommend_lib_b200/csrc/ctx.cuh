@@ -43,6 +43,8 @@ struct BookSet {
     uint32_t *uslot, *jslot, *islot;  // [maxB]  per sorted triple: DAISY_DIRECT or staging slot
     uint32_t *longs;                // rows too long for one warp (k_seg_all): [0] = #rows, [1] = #slices, then 5 words per
                                     // row (table, row, first sorted position, length, first slice), like `heavy`
+    uint32_t *counts;               // [2] staged user refs, staged item refs: the lengths of ukey_s / qkey_s when the
+                                    // bookkeeping sorted only the refs of repeated rows (step_kernels.cuh: book_kernels)
     cudaEvent_t ready, freed, copied;  // bookkeeping done / table kernels done / host triples landed (copy stream)
 };
 
@@ -142,7 +144,11 @@ struct daisy_ctx {
     // bookkeeping scratch, used on the bookkeeping stream only
     uint32_t *key_in, *val_in, *val_out;    // [3*maxB] item refs (negatives + run heads) [2*maxB]: unsorted keys/values, sorted
                                             // values; the merged sort (step_kernels.cuh) appends the user refs [maxB]
-    uint32_t *key_out;                      // [3*maxB] merged sort: sorted keys before k_slots_merged splits them
+    uint32_t *key_out;                      // [3*maxB] merged sort: sorted keys before k_slots_dup splits them
+    // merged sort of the refs of repeated rows (book_kernels): DsortState (ref_sort.cuh), the seen / dup bitmaps over
+    // ref_rows rows (user row u is bit I + u), the sort's look-back words for 3*maxB refs
+    uint32_t *ref_ws;
+    int64_t ref_rows;
     uint32_t *ukey_in, *uval_in, *uval_out; // [maxB]   user refs
     uint32_t *ikey_in, *ikey_out, *ival_in, *ival_out;  // [maxB]   (positive item, triple id), unsorted / sorted
     void *cub_tmp;
@@ -344,4 +350,10 @@ __device__ __forceinline__ float4 f4_axpy(float4 a, float s, float4 b) {
                        __fadd_rn(a.z, __fmul_rn(s, b.z)), __fadd_rn(a.w, __fmul_rn(s, b.w)));
 }
 __device__ __forceinline__ float f4_dot(float4 a, float4 b) { return a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w; }
+
+// One more reference to row r: sets its `seen` bit, and its `multi` bit if `seen` was already set.
+__device__ __forceinline__ void mark_row(uint32_t *seen, uint32_t *multi, uint32_t r) {
+    const uint32_t bit = 1u << (r & 31);
+    if (atomicOr(&seen[r >> 5], bit) & bit) atomicOr(&multi[r >> 5], bit);
+}
 #endif

@@ -186,7 +186,7 @@ static int gmf_table_phase(daisy_ctx *h, const StepPlan &pl, float *P, float *Q,
     const int NS = 64, blocksU = daisy_ceil_div(B, 8 * DAISY_SMALL_WIN), blocksQ = blocksU;
     k_seg_all<V, GradOpt, DAISY_SMALL_WIN, DAISY_SMALL_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
         P, Q, k.ukey_s, k.qkey_s, B, B, 0xFFFFFFFFu, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-        DAISY_SMALL_SLICE, k.longs, h->longs_cap, h->ticket, h->loss_part, B, loss_accum, 0);
+        DAISY_SMALL_SLICE, k.longs, h->longs_cap, h->ticket, h->loss_part, B, loss_accum, 0, nullptr);
     DAISY_LAUNCH_CHECK(h);
     k_gmf_wb<<<h->D + 1, 256, 0, s>>>(h->wpart, B, h->D, w, b, mwb, a);
     DAISY_LAUNCH_CHECK(h);

@@ -312,9 +312,7 @@ __global__ void k_owner_count(const int32_t *__restrict__ recv_ids, const uint32
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const uint32_t r = (uint32_t)ids[k];
         if (r >= rows_local) continue;
-        const uint32_t bit = 1u << (r & 31);
-        const uint32_t old = atomicOr(&seen[r >> 5], bit);
-        if (old & bit) atomicOr(&multi[r >> 5], bit);
+        mark_row(seen, multi, r);
     }
 }
 

@@ -12,6 +12,7 @@
 #include <thrust/iterator/transform_iterator.h>
 
 #include "ctx.cuh"
+#include "ref_sort.cuh"
 
 namespace {
 // ------------------------------------------------------------------------------------------------
@@ -52,9 +53,9 @@ __global__ void k_refs(const int32_t *__restrict__ triples, const uint32_t *__re
                        const uint32_t *__restrict__ sorted_i, int B, uint32_t U, uint32_t I, int C,
                        int32_t *__restrict__ st, uint32_t *__restrict__ ukey, uint32_t *__restrict__ uval,
                        uint32_t *__restrict__ qkey, uint32_t *__restrict__ qval, uint32_t *__restrict__ islot,
-                       uint32_t ukey_off, uint32_t *__restrict__ longs_hdr) {
+                       uint32_t ukey_off, uint32_t *__restrict__ longs_hdr, uint32_t *seen, uint32_t *dup) {
     int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k == 0 && longs_hdr) longs_hdr[0] = longs_hdr[1] = 0u;  // merged sort: the list is filled by k_slots_merged
+    if (k == 0 && longs_hdr) longs_hdr[0] = longs_hdr[1] = 0u;  // merged sort: the list is filled by k_slots_dup
     if (k >= B) return;
     uint32_t u, i, j;
     bool bad;
@@ -63,13 +64,20 @@ __global__ void k_refs(const int32_t *__restrict__ triples, const uint32_t *__re
     st[3 * (size_t)k + 1] = (int32_t)i;
     st[3 * (size_t)k + 2] = (int32_t)j;
     ukey[k] = u + ukey_off;  // merged sort (book_kernels): user keys follow the item keys and the sentinel
-    uval[k] = (uint32_t)k;
     qkey[k] = j;  // negative-item ref of sorted triple k
-    qval[k] = (uint32_t)k;
     const bool head = (k % C == 0) || (sorted_i[k - 1] != i);
     qkey[B + k] = head ? i : I;  // I = sentinel, sorts after every real row
-    qval[B + k] = (uint32_t)(B + k);
+    if (qval) {  // the merged sort's values are the ref positions themselves
+        uval[k] = (uint32_t)k;
+        qval[k] = (uint32_t)k;
+        qval[B + k] = (uint32_t)(B + k);
+    }
     if (!head) islot[k] = DAISY_NOT_HEAD;  // heads get their slot from k_slots_item
+    if (seen) {  // merged sort: which rows are referenced more than once (item rows, then user rows from bit I)
+        mark_row(seen, dup, I + u);
+        mark_row(seen, dup, j);
+        if (head) mark_row(seen, dup, i);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -107,40 +115,63 @@ __global__ void k_slots_item(const uint32_t *__restrict__ key, const uint32_t *_
     if (first && longs) list_long_row(key, n, p, r, 1, long_len, DAISY_SLICE, longs, longs_cap);
 }
 
-// One sort for all 3B refs (book_kernels: merged sort).  Keys: item rows [0, I), the sentinel I of the non-head positive
-// refs, user rows as I + 1 + u -- so the sorted array is [item refs | sentinels | user refs] and the user part starts at
-// position 2B exactly.  Same slots and lists as k_slots_item + k_slots_user; also splits the sorted keys into the set's
-// qkey_s [2B] and ukey_s [B] (user keys back to row ids), which is what the table kernels read.
-__global__ void k_slots_merged(const uint32_t *__restrict__ key, const uint32_t *__restrict__ val, int B, uint32_t I,
-                               uint32_t *__restrict__ qkey_s, uint32_t *__restrict__ ukey_s,
-                               uint32_t *__restrict__ uslot, uint32_t *__restrict__ jslot, uint32_t *__restrict__ islot,
-                               uint32_t *longs, int longs_cap, int long_len) {
-    const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long n2 = 2 * (long long)B, n3 = 3 * (long long)B;
-    if (p >= n3) return;
-    const uint32_t r = key[p];
-    if (p < n2) {
-        qkey_s[p] = r;
-        if (r == I) return;
-        const bool first = (p == 0) || (key[p - 1] != r);
-        const bool last = (p == n2 - 1) || (key[p + 1] != r);
-        const uint32_t slot = (first && last) ? DAISY_DIRECT : (uint32_t)p;
-        const uint32_t v = val[p];
-        if (v < (uint32_t)B)
-            jslot[v] = slot;
+// Merged sort (book_kernels): ref x of the 3B refs k_refs wrote -- negatives [0, B), run heads [B, 2B) (key I: not a
+// head), users [2B, 3B) (key I + 1 + u) -- goes into the sort only if its row has another ref in the same table.  A ref
+// whose row has none is DIRECT, and is settled here.
+struct BprRefSrc {
+    const uint32_t *key, *dup;
+    int B;
+    uint32_t I;
+    uint32_t *jslot, *islot, *uslot;
+    __device__ __forceinline__ bool operator()(int x, uint32_t &k) const {
+        const uint32_t r = key[x];
+        if (r == I) return false;
+        const uint32_t bit = r < I ? r : r - 1u;
+        if (dup[bit >> 5] >> (bit & 31) & 1u) {
+            k = r;
+            return true;
+        }
+        if (x < B)
+            jslot[x] = DAISY_DIRECT;
+        else if (x < 2 * B)
+            islot[x - B] = DAISY_DIRECT;
         else
-            islot[v - B] = slot;
-        if (first && longs) list_long_row(key, (int)n2, (int)p, r, 1, long_len, DAISY_SLICE, longs, longs_cap);
-    } else {
-        const int q = (int)(p - n2);
-        const uint32_t *ukey = key + n2;
-        ukey_s[q] = r - (I + 1u);
-        const bool first = (q == 0) || (ukey[q - 1] != r);
-        const bool last = (q == B - 1) || (ukey[q + 1] != r);
-        uslot[val[p]] = (first && last) ? DAISY_DIRECT : (uint32_t)q;
-        if (first && longs) {  // the list holds row ids: search the run in the offset keys, record the row itself
-            if (q + long_len < B && ukey[q + long_len] == r) {
-                int lo = q + long_len, hi = B - 1;
+            uslot[x - 2 * B] = DAISY_DIRECT;
+        return false;
+    }
+};
+
+// The sorted refs of repeated rows: ss->n of them, the ss->n_lo item refs first (keys < I), then the user refs (keys
+// I + 1 + u), each row's refs in their order among the 3B.  Every one of them shares its row, so it is staged at its
+// position in its table's part.  Splits the keys into the set's qkey_s / ukey_s (user keys back to row ids), which is
+// what the table kernels read, lists the rows longer than long_len and records both counts for k_seg_all.
+__global__ void k_slots_dup(const uint32_t *__restrict__ key, const uint32_t *__restrict__ val, const DsortState *ss, int B,
+                            uint32_t I, uint32_t *__restrict__ qkey_s, uint32_t *__restrict__ ukey_s,
+                            uint32_t *__restrict__ uslot, uint32_t *__restrict__ jslot, uint32_t *__restrict__ islot,
+                            uint32_t *__restrict__ counts, uint32_t *longs, int longs_cap, int long_len) {
+    const int n = (int)ss->n, nq = (int)ss->n_lo, nu = n - nq;
+    const int p0 = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p0 == 0) {
+        counts[0] = (uint32_t)nu;
+        counts[1] = (uint32_t)nq;
+    }
+    for (int p = p0; p < n; p += gridDim.x * blockDim.x) {
+        const uint32_t r = key[p], v = val[p];
+        if (p < nq) {
+            qkey_s[p] = r;
+            if (v < (uint32_t)B)
+                jslot[v] = (uint32_t)p;
+            else
+                islot[v - B] = (uint32_t)p;
+            if (p == 0 || key[p - 1] != r) list_long_row(key, nq, p, r, 1, long_len, DAISY_SLICE, longs, longs_cap);
+        } else {
+            const int q = p - nq;
+            const uint32_t *ukey = key + nq;
+            ukey_s[q] = r - (I + 1u);
+            uslot[v - 2u * (uint32_t)B] = (uint32_t)q;
+            if ((q == 0 || ukey[q - 1] != r) && q + long_len < nu && ukey[q + long_len] == r) {
+                // a long user row: the list holds row ids, so search the run in the offset keys and record the row
+                int lo = q + long_len, hi = nu - 1;
                 while (lo < hi) {
                     const int mid = (int)(((long long)lo + hi + 1) >> 1);
                     if (ukey[mid] == r) lo = mid; else hi = mid - 1;
@@ -755,6 +786,7 @@ __device__ __forceinline__ void block_sort_words(uint32_t (&keys)[IPT], int ipt,
 }
 
 #define DAISY_SMALL_HIST_WORDS (32 * 513)
+#define DAISY_SEG_WIN_BLOCKS 8  // general path, merged sort: k_seg_all's window blocks per table and SM (they stride)
 #define DAISY_SMALL_WIN 8       // sorted refs per warp of k_seg_all
 #define DAISY_SMALL_SLICE 16   // contributions per slice of a long row (k_seg_all): short, so that a hot row's
                                // sum is spread over many warps on many SMs and is not a latency chain
@@ -1285,7 +1317,8 @@ __global__ void DAISY_SEG_BOUNDS k_seg_all(const float *__restrict__ P, const fl
                                                   float *__restrict__ stage2, int D4, Opt opt, int NS, int blocksU,
                                                   int blocksQ, int long_len, const uint32_t *__restrict__ longs,
                                                   int longs_cap, uint32_t *ticket, const float *__restrict__ loss_part,
-                                                  int n_part, double *loss_accum, int ilvQ) {
+                                                  int n_part, double *loss_accum, int ilvQ,
+                                                  const uint32_t *__restrict__ counts) {
     const int b = blockIdx.x, wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const unsigned FULL = 0xffffffffu;
     if (b >= NS + blocksU + blocksQ) {  // fixed-order reduction of the per-warp loss partials (double accumulation)
@@ -1314,8 +1347,13 @@ __global__ void DAISY_SEG_BOUNDS k_seg_all(const float *__restrict__ P, const fl
             const int per = blocksQ / ilvQ;
             w = (w % ilvQ) * per + w / ilvQ;
         }
-        seg_window<V, Opt, WIN>((long long)w * 8 + wid, tbl, tbl ? Q : P, tbl ? qkey_s : ukey_s,
-                                tbl ? nQ : B, tbl ? q_sentinel : 0xFFFFFFFFu, tbl ? stageQ : stageU, D4, opt, long_len);
+        // counts (merged sort of the refs of repeated rows): the ref counts of the two tables are known on the device
+        // only, and the grid may hold fewer windows than there are -- a table's blocks stride over its windows
+        const int n = counts ? (int)counts[tbl] : (tbl ? nQ : B);
+        const long long stride = 8LL * (tbl ? blocksQ : blocksU);
+        for (long long ww = (long long)w * 8 + wid; ww * WIN < n; ww += stride)
+            seg_window<V, Opt, WIN>(ww, tbl, tbl ? Q : P, tbl ? qkey_s : ukey_s, n, tbl ? q_sentinel : 0xFFFFFFFFu,
+                                    tbl ? stageQ : stageU, D4, opt, long_len);
         return;
     }
     const int count = min((int)longs[0], longs_cap);
@@ -1448,8 +1486,8 @@ static int bits_for(uint64_t max_value) {  // number of low bits needed to repre
 // merged sort of the 3B refs (book_kernels): worth it when it costs no more element-passes than the two separate sorts
 // (it always saves the fixed cost of one sort: histogram + scan launches and one wave per pass)
 static bool use_merged_sort(const daisy_ctx *h, uint32_t U, uint32_t I) {
-    if (h->merged_sort == 0) return false;
-    if ((uint64_t)U + I > 0xFFFFFFF0ull || 3 * h->maxB >= (1ll << 31)) return false;
+    if (h->merged_sort == 0 || !h->ref_ws) return false;
+    if ((uint64_t)U + I > 0xFFFFFFF0ull || (int64_t)U + I > h->ref_rows) return false;
     if (h->merged_sort == 1) return true;
     const int pu = (bits_for(U - 1) + 7) / 8, pq = (bits_for(I) + 7) / 8, pm = (bits_for((uint64_t)I + U) + 7) / 8;
     return 3 * pm <= pu + 2 * pq;
@@ -1557,6 +1595,7 @@ struct StepPlan {
     const float *const *jsrc, *const *isrc;  // row-sharded step only (else null)
     bool small;           // small-batch path: k_small_book / C = 1 / k_seg_all
     int ilv;              // row-sharded step: chunk interleave of the main kernel (MainArgs::ilv), else 0
+    const uint32_t *counts;  // merged sort: the set's device-side ref counts (BookSet::counts) for k_seg_all, else null
 };
 
 // Does a batch of B triples take the small-batch path?  Its refs must pack into 32 bits: row bits (of the VALUE U
@@ -1585,27 +1624,38 @@ static int book_kernels(daisy_ctx *h, BookSet &k, const StepPlan &pl, const int3
     h->launches += 4;
     phase_mark(h, PH_SORT_I, s);
     // refs
-    // One sort for all 3B refs when the table is not sharded and the combined key space costs no extra radix passes
-    // (config 4: 10 M users + 2 M items = 24 bits = 3 passes over 3 M pairs, instead of 3 over 1 M + 3 over 2 M, and
-    // 7 launches instead of 14): bit-identical products, the sort is stable and the refs enter it in the same order.
-    if (!sh && use_merged_sort(h, U, I)) {
+    // One sort for the user and item refs when the table is not sharded and the combined key space costs no extra radix
+    // passes (config 4: 10 M users + 2 M items = 24 bits = 3 passes).  Only the refs of rows referenced more than once
+    // in their table go into it: k_refs marks every row in two bitmaps (seen / dup), the compaction settles every other
+    // ref as DIRECT and keeps the rest in their order (negatives, run heads, users), and ref_sort.cuh sorts those --
+    // about 0.7 M of the 3 M refs of a config-4 batch -- with a count that stays on the device.  The sort is stable and
+    // the refs of a row keep their order, so every row is summed in the same order as by two full sorts.
+    if (pl.counts) {
+        uint32_t *ws = h->ref_ws;
+        DsortState *ss = reinterpret_cast<DsortState *>(ws);
+        const size_t bm_words = (size_t)((h->ref_rows + 31) / 32);
+        uint32_t *seen = ws + sizeof(DsortState) / 4, *dup = seen + bm_words, *status = dup + bm_words;
+        DAISY_CUDA(cudaMemsetAsync(ws, 0, (sizeof(DsortState) / 4 + 2 * bm_words + dsort_tiles(3 * (int64_t)B)) * sizeof(uint32_t), bs));
         k_refs<<<daisy_ceil_div(B, T), T, 0, bs>>>(triples, h->ival_out, h->ikey_out, B, U, I, C, k.st, h->key_in + 2 * (size_t)B,
-                                                   h->val_in + 2 * (size_t)B, h->key_in, h->val_in, k.islot, I + 1u, k.longs);
+                                                   nullptr, h->key_in, nullptr, k.islot, I + 1u, k.longs, seen, dup);
         DAISY_LAUNCH_CHECK(h);
         phase_mark(h, PH_REFS, s);
-        tmp = h->cub_tmp_bytes;
-        DAISY_CUDA(cub::DeviceRadixSort::SortPairs(h->cub_tmp, tmp, h->key_in, h->key_out, h->val_in, h->val_out, 3 * B, 0,
-                                                   bits_for((uint64_t)I + U), bs));
-        h->launches += 4;
+        uint32_t *skey, *sval;
+        const BprRefSrc src{h->key_in, dup, B, I, k.jslot, k.islot, k.uslot};
+        h->launches += dsort_launch(src, 3 * B, I, bits_for((uint64_t)I + U), h->key_out, h->val_out, h->key_in, h->val_in,
+                                    ss, status, 2 * h->num_sms, bs, &skey, &sval) - 1;
+        DAISY_LAUNCH_CHECK(h);
         phase_mark(h, PH_SORT_U, s);
         phase_mark(h, PH_SORT_Q, s);
-        k_slots_merged<<<daisy_ceil_div(3 * (int64_t)B, T), T, 0, bs>>>(h->key_out, h->val_out, B, I, k.qkey_s, k.ukey_s, k.uslot,
-                                                                        k.jslot, k.islot, k.longs, h->longs_cap, h->heavy_len);
+        const int gs = daisy_ceil_div(3 * (int64_t)B, T);
+        k_slots_dup<<<gs < 8 * h->num_sms ? gs : 8 * h->num_sms, T, 0, bs>>>(skey, sval, ss, B, I, k.qkey_s, k.ukey_s, k.uslot,
+                                                                          k.jslot, k.islot, k.counts, k.longs, h->longs_cap,
+                                                                          h->heavy_len);
         DAISY_LAUNCH_CHECK(h);
         return DAISY_OK;
     }
     k_refs<<<daisy_ceil_div(B, T), T, 0, bs>>>(triples, h->ival_out, h->ikey_out, B, U, I, C, k.st, h->ukey_in,
-                                               h->uval_in, h->key_in, h->val_in, k.islot, 0u, nullptr);
+                                               h->uval_in, h->key_in, h->val_in, k.islot, 0u, nullptr, nullptr, nullptr);
     DAISY_LAUNCH_CHECK(h);
     phase_mark(h, PH_REFS, s);
     tmp = h->cub_tmp_bytes;
@@ -1675,11 +1725,13 @@ static int book_phase(daisy_ctx *h, StepPlan &pl, const int32_t *triples, int64_
     pl.B = B; pl.C = C; pl.U = U; pl.I = I; pl.piped = piped; pl.bs = bs; pl.s = s;
     pl.set = h->book_idx;
     pl.small = small;
+    pl.counts = nullptr;
     pl.jsrc = sh ? sh->set[pl.set].jsrc : nullptr;
     pl.isrc = sh ? sh->set[pl.set].isrc : nullptr;
     pl.ilv = sh ? sh->ilv : 0;
     BookSet &k = h->book[h->book_idx];
     pl.k = &k;
+    if (!sh && !small && use_merged_sort(h, U, I)) pl.counts = k.counts;
     h->book_idx = (h->book_idx + 1) % DAISY_NSETS;
     if (h->timing == 2) {
         if (h->ev_pending) {  // fold the previous step's phase times in
@@ -1865,19 +1917,24 @@ static int table_phase_v(daisy_ctx *h, const StepPlan &pl, const float *P, const
             blocksU = daisy_ceil_div(B, 8 * DAISY_SMALL_WIN), blocksQ = daisy_ceil_div(2 * B, 8 * DAISY_SMALL_WIN);
             k_seg_all<V, Opt, DAISY_SMALL_WIN, DAISY_SMALL_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
                 P, Q, k.ukey_s, k.qkey_s, B, 2 * B, 0xFFFFFFFFu, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-                DAISY_SMALL_SLICE, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, 0);
-        } else if (h->seg_win == 16) {  // DAISY_SEG_WIN: sorted refs per warp of the window blocks (general path)
-            blocksU = daisy_ceil_div(B, 8 * 16), blocksQ = daisy_ceil_div(2 * (int64_t)B, 8 * 16);
-            if (ilvQ) blocksQ = daisy_ceil_div(blocksQ, ilvQ) * ilvQ;
-            k_seg_all<V, Opt, 16, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
-                P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-                h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ);
+                DAISY_SMALL_SLICE, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, 0, nullptr);
         } else {
-            blocksU = daisy_ceil_div(B, 8 * 32), blocksQ = daisy_ceil_div(2 * (int64_t)B, 8 * 32);
+            const int win = h->seg_win == 16 ? 16 : 32;  // DAISY_SEG_WIN: sorted refs per warp of the window blocks
+            blocksU = daisy_ceil_div(B, 8 * win), blocksQ = daisy_ceil_div(2 * (int64_t)B, 8 * win);
             if (ilvQ) blocksQ = daisy_ceil_div(blocksQ, ilvQ) * ilvQ;
-            k_seg_all<V, Opt, 32, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
-                P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-                h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ);
+            if (pl.counts) {  // the merged sort holds only the refs of repeated rows, a count known on the device only
+                const int cap = DAISY_SEG_WIN_BLOCKS * h->num_sms;
+                if (blocksU > cap) blocksU = cap;
+                if (blocksQ > cap) blocksQ = cap;
+            }
+            if (win == 16)
+                k_seg_all<V, Opt, 16, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
+                    P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
+                    h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ, pl.counts);
+            else
+                k_seg_all<V, Opt, 32, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
+                    P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
+                    h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ, pl.counts);
         }
         DAISY_LAUNCH_CHECK(h);
         for (int ph = PH_SEG_U; ph <= PH_LOSS; ++ph) phase_mark(h, ph, s);
