@@ -52,10 +52,10 @@ def _stale(target, deps):
 def build(force=False, verbose=False):
     """Compile every csrc/*.cu to an object (only the stale ones) and link the shared library.
 
-    Experiments (DESIGN.md section 11): DAISY_NVCC_EXTRA="-DDAISY_SEG_MIN_BLOCKS=2 -DDAISY_SEG_COMBINE_TILE=4" with
-    DAISY_LIB_VARIANT=seg2 builds libdaisy_b200_seg2.so from objects under csrc/_obj_seg2/ next to the default library,
-    which is left alone; a process started with DAISY_LIB_VARIANT=seg2 loads that one (_lib.py), so both travel to the
-    GPU box in one snapshot and one call can measure them side by side."""
+    Experiments (DESIGN.md section 11): DAISY_NVCC_EXTRA="-maxrregcount=64" with DAISY_LIB_VARIANT=r64 builds
+    libdaisy_b200_r64.so from objects under csrc/_obj_r64/ next to the default library, which is left alone; a process
+    started with DAISY_LIB_VARIANT=r64 loads that one (_lib.py), so both travel to the GPU box in one snapshot and one
+    call can measure them side by side."""
     nvcc = _nvcc()
     extra = shlex.split(os.environ.get("DAISY_NVCC_EXTRA", ""))
     variant = os.environ.get("DAISY_LIB_VARIANT", "")

@@ -108,14 +108,12 @@ extern "C" int daisy_create(daisy_handle_t *out, int device, int64_t user_num, i
     if (h->main_stages < 0) h->main_stages = 0;
     if (h->main_stages > 16) h->main_stages = 16;
     h->inputs_ready = 0;
-    h->seg_win = env_int("DAISY_SEG_WIN", 32) == 16 ? 16 : 32;
     h->mid_max = env_int("DAISY_MID_MAX", 65536);  // measured: above ~100 k triples the general pipeline (graph-replayed) is faster
     if (h->mid_max < 0) h->mid_max = 0;
     if (h->mid_max > h->mid_cap) h->mid_max = h->mid_cap;
     h->graph_max_b = env_int("DAISY_GRAPH_MAX_B", 262144);
     if (h->graph_max_b < 0) h->graph_max_b = 0;
     h->merged_sort = env_int("DAISY_MERGED_SORT", -1);
-    h->main_max_blocks = env_int("DAISY_MAIN_MAX_BLOCKS", 0);
     h->small_max = env_int("DAISY_SMALL_MAX", DAISY_SMALL_CAP);
     if (h->small_max < 0) h->small_max = 0;
     if (h->small_max > DAISY_SMALL_CAP) h->small_max = DAISY_SMALL_CAP;
@@ -174,18 +172,7 @@ extern "C" int daisy_create(daisy_handle_t *out, int device, int64_t user_num, i
         // bandwidth-bound kernels of step n are still dispatching blocks
         int prio_lo = 0, prio_hi = 0;
         cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-        cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking,
-                                     env_int("DAISY_BOOK_LOW_PRIORITY", 0) ? prio_lo : prio_hi);
-        // DAISY_BOOK_SMS = n > 0: the bookkeeping stream gets n SMs of its own and the table kernels the rest
-        // (partition.cu); a driver that cannot partition leaves the shared-SM pipeline in place
-        if (B > 0 && h->pipeline && env_int("DAISY_BOOK_SMS", 0) > 0) {
-            if (daisy_partition_create(h, env_int("DAISY_BOOK_SMS", 0)) == DAISY_OK && h->part_ok) {
-                cudaStreamDestroy(h->side_stream);
-                h->side_stream = h->part_book_stream;
-            } else if (env_int("DAISY_BOOK_SMS_REQUIRED", 0)) {
-                rc = DAISY_EUNSUPPORTED;
-            }
-        }
+        cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking, prio_hi);
         cudaEventCreateWithFlags(&h->ev_call, cudaEventDisableTiming);
         for (int i = 0; i < DAISY_NSETS; ++i) {
             cudaEventCreateWithFlags(&h->book[i].ready, cudaEventDisableTiming);
@@ -213,7 +200,7 @@ extern "C" int daisy_destroy(daisy_handle_t h) {
     daisy_shard_free(h);
     void *ptrs[] = {h->triples, h->key_in, h->val_in, h->val_out, h->ukey_in, h->uval_in, h->uval_out, h->ikey_in,
                     h->ikey_out, h->ival_in, h->ival_out, h->stageU, h->stageQ, h->stage2, h->loss_part, h->key_out,
-                    h->err, h->cub_tmp, h->ticket, h->mid_buf, h->gradP, h->gradQ, h->wpart, h->scores, h->sel_hist, h->own_key, h->own_key_s, h->own_val, h->own_val_s,
+                    h->err, h->cub_tmp, h->ticket, h->mid_buf, h->gradP, h->gradQ, h->wpart, h->scores, h->own_key, h->own_key_s, h->own_val, h->own_val_s,
                     h->own_tmp, h->ref_ws};
     for (void *p : ptrs)
         if (p) cudaFree(p);
@@ -233,10 +220,6 @@ extern "C" int daisy_destroy(daisy_handle_t h) {
     if (h->pool_state == 1) cudaMemPoolDestroy(h->pool);
     if (h->err_host) cudaFreeHost(h->err_host);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->part_ok) {
-        h->side_stream = nullptr;  // it is the partition's bookkeeping stream
-        daisy_partition_destroy(h);
-    }
     if (h->side_stream) cudaStreamDestroy(h->side_stream);
     if (h->ev_call) cudaEventDestroy(h->ev_call);
     for (int i = 0; i <= PH_COUNT; ++i)

@@ -173,7 +173,6 @@ struct daisy_ctx {
     // full-catalogue top-K workspace (grown on demand by daisy_topk_full)
     float *scores;          // [tile_users, item_num] score tile
     size_t scores_cap;      // floats
-    unsigned *sel_hist;     // unused placeholder for a fused histogram (kept null)
 
     // tuning (env overridable, see api.cu)
     int chunk;       // max positive-item run length handled by one warp in the main kernel (0 = auto)
@@ -183,13 +182,6 @@ struct daisy_ctx {
     float *gradP, *gradQ;  // [U, D], [I, D] dense gradient buffers of the GMF step (allocated on first use, kept zero between steps)
     float *wpart;    // [maxB, D + 1] per-sample contributions to the predict layer's gradient (GMF step)
     int merged_sort; // general path: ONE radix sort for user + item refs: 1 always, 0 never, -1 (default) when it costs no extra passes
-    int main_max_blocks;  // experiment (DAISY_MAIN_MAX_BLOCKS): resident blocks per SM of the TMA main kernel capped through its shared-memory request
-    // SM partitioning (partition.cu): bookkeeping stream on part_book_sms SMs, table kernels on the rest
-    int part_ok, part_book_sms, part_main_sms;
-    void *part_green[2];
-    cudaStream_t part_book_stream, part_main_stream;
-    cudaEvent_t part_ev_in, part_ev_out;
-    int seg_win;     // sorted refs per warp of k_seg_all's window blocks in the general path: 32 (default) or 16
     int small_max;   // batches up to this many triples take the 3-launch small-batch path (0 = never; <= DAISY_SMALL_CAP)
     int64_t mid_max; // ... and up to this many the same path with k_mid_book (0 = never; <= mid_cap)
     int64_t mid_cap; // min(maxB, 131072): what mid_buf is sized for
@@ -230,8 +222,6 @@ struct daisy_ctx {
 
 void daisy_set_error(const char *fmt, ...);
 void daisy_shard_free(daisy_ctx *h);  // shard.cu
-int daisy_partition_create(daisy_ctx *h, int book_sms);  // partition.cu
-void daisy_partition_destroy(daisy_ctx *h);
 
 #define DAISY_CUDA(call)                                                                     \
     do {                                                                                     \

@@ -320,8 +320,8 @@ __global__ void k_owner_count(const int32_t *__restrict__ recv_ids, const uint32
 // sender's excl array).  The sender then stores the updated row straight into the owner's q instead of pushing a sum
 // the owner would have to read, add and write back.  What stays with the owner are the rows SHARED between ranks: every
 // such row gets a SLOT (claimed once through a third bitmap) with one cell per sender, filled by k_owner_pairs, so that
-// the owner's kernel can walk the shared rows directly; the shared entries are also listed per sender for the
-// pass-per-sender variant (order inside a list is arbitrary and does not matter: a sender's entries name distinct rows).
+// the owner's kernel can walk the shared rows directly; k_owner_pairs reads the shared entries from per-sender lists
+// (order inside a list is arbitrary and does not matter: a sender's entries name distinct rows).
 __global__ void k_owner_classify(const int32_t *__restrict__ recv_ids, const uint32_t *__restrict__ recv_cnt, size_t cap,
                                  uint32_t rows_local, const uint32_t *__restrict__ multi, int me, ShardPeers peers,
                                  uint32_t *__restrict__ shared_idx, uint32_t *__restrict__ shared_cnt,
@@ -415,100 +415,6 @@ __global__ void k_shard_barrier(ShardPeers peers, int me, int G, uint32_t epoch,
     __threadfence_system();
 }
 
-// Owner side.  Region s of recv_ids holds the ascending, duplicate-free local row ids sender s pushed sums for
-// (recv_cnt[s] of them), recv_g the sums.  One lane per entry: it is the row's LEADER if no lower-ranked sender
-// pushed the same row (binary searches); the warp then handles its leaders one at a time, adding the senders'
-// sums in rank order and updating the row once.
-template <int V>
-__global__ void __launch_bounds__(256) k_owner_merge(float *__restrict__ Q, const float *__restrict__ recv_g,
-                                                      const int32_t *__restrict__ recv_ids,
-                                                      const uint32_t *__restrict__ recv_cnt, int G, size_t cap, int D4,
-                                                      float alpha, uint32_t rows_local, int *err) {
-    const unsigned FULL = 0xffffffffu;
-    const uint32_t NONE = 0xFFFFFFFFu;
-    const int lane = threadIdx.x & 31;
-    const uint32_t warp = (uint32_t)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
-    const uint32_t nwarps = (uint32_t)((gridDim.x * (size_t)blockDim.x) >> 5);
-    uint32_t cnt_l = (lane < G) ? recv_cnt[lane] : 0u;
-    if (cnt_l > cap) {  // cannot happen (a sender has at most 2*maxB = cap distinct rows); never read out of bounds
-        atomicOr(&err[0], 32);
-        cnt_l = (uint32_t)cap;
-    }
-    uint32_t total = 0;
-    for (int s = 0; s < G; ++s) total += (__shfl_sync(FULL, cnt_l, s) + 31u) >> 5;
-    bool act[V];
-#pragma unroll
-    for (int v = 0; v < V; ++v) act[v] = (lane + 32 * v) < D4;
-
-    for (uint32_t task = warp; task < total; task += nwarps) {
-        int s = 0;
-        uint32_t rem = task;
-        while (true) {
-            const uint32_t ch = (__shfl_sync(FULL, cnt_l, s) + 31u) >> 5;
-            if (rem < ch) break;
-            rem -= ch;
-            ++s;
-        }
-        const uint32_t n_s = __shfl_sync(FULL, cnt_l, s);
-        const uint32_t k = rem * 32u + lane;
-        const bool valid = k < n_s;
-        uint32_t r = valid ? (uint32_t)recv_ids[(size_t)s * cap + k] : NONE;
-        bool leader = valid;
-        if (valid && r >= rows_local) {
-            atomicOr(&err[0], 1);
-            leader = false;
-        }
-        uint32_t pos[DAISY_MAX_RANKS];
-#pragma unroll
-        for (int sp = 0; sp < DAISY_MAX_RANKS; ++sp) {
-            pos[sp] = NONE;
-            if (sp < G && sp != s) {  // warp-uniform
-                const uint32_t n2 = __shfl_sync(FULL, cnt_l, sp);
-                const int32_t *ids2 = recv_ids + (size_t)sp * cap;
-                uint32_t lo = 0, hi = n2;
-                while (__any_sync(FULL, lo < hi)) {
-                    if (lo < hi) {
-                        const uint32_t mid = (lo + hi) >> 1;
-                        if ((uint32_t)ids2[mid] < r) lo = mid + 1; else hi = mid;
-                    }
-                }
-                const bool found = valid && lo < n2 && (uint32_t)ids2[lo] == r;
-                if (found) {
-                    if (sp < s) leader = false; else pos[sp] = lo;
-                }
-            }
-        }
-        unsigned todo = __ballot_sync(FULL, leader);
-        while (todo) {
-            const int b = __ffs(todo) - 1;
-            todo &= todo - 1;
-            const uint32_t row = __shfl_sync(FULL, r, b);
-            float4 acc[V];
-            const size_t own = ((size_t)s * cap + rem * 32u + b) * D4;
-#pragma unroll
-            for (int v = 0; v < V; ++v) acc[v] = act[v] ? ld_stream(recv_g, own + lane + 32 * v) : f4_zero();
-#pragma unroll
-            for (int sp = 0; sp < DAISY_MAX_RANKS; ++sp) {
-                const uint32_t pp = __shfl_sync(FULL, pos[sp], b);
-                if (pp != NONE) {  // warp-uniform; sp > s ascending = sender-rank order
-                    const size_t at = ((size_t)sp * cap + pp) * D4;
-#pragma unroll
-                    for (int v = 0; v < V; ++v)
-                        if (act[v]) acc[v] = f4_add(acc[v], ld_stream(recv_g, at + lane + 32 * v));
-                }
-            }
-#pragma unroll
-            for (int v = 0; v < V; ++v)
-                if (act[v]) {
-                    const size_t e = (size_t)row * D4 + lane + 32 * v;
-                    const float4 old = ld_row(Q, e);
-                    st_row(Q, e, make_float4(fmaf(alpha, acc[v].x, old.x), fmaf(alpha, acc[v].y, old.y),
-                                             fmaf(alpha, acc[v].z, old.z), fmaf(alpha, acc[v].w, old.w)));
-                }
-        }
-    }
-}
-
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // Arena layout (identical on every rank): a function of (dim, max_batch, world, item_num_global) only.
@@ -551,24 +457,21 @@ static void launch_fetch(daisy_ctx *h, const ShardSet &ss, cudaStream_t s) {
     k_shard_fetch<V, 4><<<h->num_sms * 4, 256, 0, s>>>(ss.src, ss.multi, ss.owner_off, sh->world, sh->cache, h->D / 4, sh->ilv);
 }
 
-// Owner side, default: ONE PASS PER SENDER, in sender-rank order.  A sender's id list is duplicate-free, so the
-// entries of one region touch distinct rows and a pass is a plain streaming read-modify-write (R entries in flight per
-// warp); passes follow each other on the stream, which fixes the order in which a row shared by several senders
-// receives their sums => deterministic, no membership searches at all.  (k_owner_merge, the single-pass variant that
-// finds every row's senders by binary search, cost 0.57 ms at 8 ranks -- 7 x 17 dependent L2 loads per entry; it is
-// kept behind DAISY_OWNER_MERGE=1.)
+// Owner side with the exclusive-row bypass off: ONE PASS PER SENDER, in sender-rank order.  A sender's id list is
+// duplicate-free, so the entries of one region touch distinct rows and a pass is a plain streaming read-modify-write
+// (R entries in flight per warp); passes follow each other on the stream, which fixes the order in which a row shared
+// by several senders receives their sums => deterministic, no membership searches at all.  (A single-pass merge that
+// found every row's senders by binary search cost 0.57 ms at 8 ranks -- 7 x 17 dependent L2 loads per entry; it was
+// measured and removed, DESIGN.md section 7.)
 template <int V, int R>
 __global__ void __launch_bounds__(256) k_owner_add(float *__restrict__ Q, const float *__restrict__ recv_g,
                                                     const int32_t *__restrict__ recv_ids,
                                                     const uint32_t *__restrict__ recv_cnt_s, size_t cap, int D4, float alpha,
-                                                    uint32_t rows_local, int *err, const uint32_t *__restrict__ list,
-                                                    const uint32_t *__restrict__ list_cnt) {
-    // list != null (exclusive-row bypass live this step): an entry whose row no other rank referenced has already been
-    // written, updated, by its sender -- only the listed entries (rows shared between ranks) are added here
+                                                    uint32_t rows_local, int *err) {
     const int lane = threadIdx.x & 31;
     const uint32_t warp = (uint32_t)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
     const uint32_t nwarps = (uint32_t)((gridDim.x * (size_t)blockDim.x) >> 5);
-    uint32_t n = list ? *list_cnt : *recv_cnt_s;
+    uint32_t n = *recv_cnt_s;
     if (n > cap) {  // cannot happen (a sender has at most 2*maxB = cap distinct rows); never read out of bounds
         if (threadIdx.x == 0 && blockIdx.x == 0) atomicOr(&err[0], 32);
         n = (uint32_t)cap;
@@ -578,14 +481,12 @@ __global__ void __launch_bounds__(256) k_owner_add(float *__restrict__ Q, const 
     for (int v = 0; v < V; ++v) act[v] = (lane + 32 * v) < D4;
     for (uint32_t k0 = warp * R; k0 < n; k0 += nwarps * R) {
         float4 g[R][V], old[R][V];
-        uint32_t row[R], ent[R];
+        uint32_t row[R];
 #pragma unroll
         for (int jj = 0; jj < R; ++jj) {
             row[jj] = 0xFFFFFFFFu;
-            ent[jj] = 0;
             if (k0 + jj < n) {
-                ent[jj] = list ? list[k0 + jj] : k0 + jj;
-                row[jj] = (uint32_t)recv_ids[ent[jj]];
+                row[jj] = (uint32_t)recv_ids[k0 + jj];
                 if (row[jj] >= rows_local) {
                     if (lane == 0) atomicOr(&err[0], 1);
                     row[jj] = 0xFFFFFFFFu;
@@ -598,7 +499,7 @@ __global__ void __launch_bounds__(256) k_owner_add(float *__restrict__ Q, const 
 #pragma unroll
                 for (int v = 0; v < V; ++v)
                     if (act[v]) {
-                        g[jj][v] = ld_stream(recv_g, (size_t)ent[jj] * D4 + lane + 32 * v);
+                        g[jj][v] = ld_stream(recv_g, (size_t)(k0 + jj) * D4 + lane + 32 * v);
                         old[jj][v] = ld_row(Q, (size_t)row[jj] * D4 + lane + 32 * v);
                     }
             }
@@ -665,17 +566,9 @@ template <int V>
 static void launch_merge(daisy_ctx *h, float alpha, cudaStream_t s) {
     daisy_shard *sh = h->sh;
     const int me = sh->rank;
-    static const int single_pass = getenv("DAISY_OWNER_MERGE") && atoi(getenv("DAISY_OWNER_MERGE")) == 1;
-    if (single_pass) {
-        k_owner_merge<V><<<h->num_sms * 8, 256, 0, s>>>(sh->peers.q[me], sh->peers.recv_g[me], sh->peers.recv_ids[me],
-                                                        sh->peers.recv_cnt[me], sh->world, (size_t)sh->cap, h->D / 4, alpha,
-                                                        (uint32_t)h->I, h->err);
-        return;
-    }
     constexpr int R = V == 1 ? 4 : 2;
     const size_t cap = (size_t)sh->cap;
-    static const int shared_passes = getenv("DAISY_OWNER_SHARED_PASSES") && atoi(getenv("DAISY_OWNER_SHARED_PASSES")) == 1;
-    if (sh->classified && !shared_passes) {
+    if (sh->classified) {
         k_owner_add_slots<V><<<h->num_sms * 8, 256, 0, s>>>(sh->peers.q[me], sh->peers.recv_g[me], sh->slot_row, sh->pairs,
                                                             sh->slot_n, sh->max_slots, sh->world, cap, h->D / 4, alpha);
         return;
@@ -684,8 +577,7 @@ static void launch_merge(daisy_ctx *h, float alpha, cudaStream_t s) {
         k_owner_add<V, R><<<h->num_sms * 8, 256, 0, s>>>(sh->peers.q[me], sh->peers.recv_g[me] + (size_t)snd * cap * h->D,
                                                          sh->peers.recv_ids[me] + (size_t)snd * cap,
                                                          sh->peers.recv_cnt[me] + snd, cap, h->D / 4, alpha, (uint32_t)h->I,
-                                                         h->err, sh->classified ? sh->shared_idx + (size_t)snd * cap : nullptr,
-                                                         sh->shared_cnt + snd);
+                                                         h->err);
         if (snd + 1 < sh->world) h->launches++;
     }
 }
@@ -946,10 +838,9 @@ extern "C" int daisy_shard_init(daisy_handle_t h, int rank, int world, int64_t i
     ok = ok && cudaMalloc((void **)&sh->slot_row, (size_t)sh->max_slots * sizeof(uint32_t)) == cudaSuccess;
     ok = ok && cudaMalloc((void **)&sh->pairs, (size_t)sh->max_slots * world * sizeof(uint32_t)) == cudaSuccess;
     sh->plan = new StepPlan();
-    {   // exclusive-row bypass (on by default; the single-pass owner merge does not know about it)
+    {   // exclusive-row bypass (on by default)
         const char *v = getenv("DAISY_SHARD_BYPASS");
-        const char *m = getenv("DAISY_OWNER_MERGE");
-        sh->bypass = ((v && *v) ? atoi(v) != 0 : 1) && !(m && atoi(m) == 1);
+        sh->bypass = (v && *v) ? atoi(v) != 0 : 1;
     }
     for (int i = 0; i < DAISY_NSETS && ok; ++i) {
         ok = ok && cudaMalloc((void **)&sh->set[i].uniq_gid, cap * sizeof(uint32_t)) == cudaSuccess;

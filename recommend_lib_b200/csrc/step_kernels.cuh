@@ -401,15 +401,8 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
                  : "memory");
 }
 
-// DAISY_MAIN_MIN_BLOCKS (build-time experiment, tools/build_variants.sh): minimum resident blocks per SM the compiler must
-// allow -- 5 caps the kernel at 51 registers (default build: 62 registers at V = 1, 4 blocks per SM by registers).
-#ifndef DAISY_MAIN_MIN_BLOCKS
-#define DAISY_MAIN_BOUNDS __launch_bounds__(256)
-#else
-#define DAISY_MAIN_BOUNDS __launch_bounds__(256, (V == 1 ? DAISY_MAIN_MIN_BLOCKS : 1))
-#endif
 template <int V, class Opt, bool PTR>
-__global__ void DAISY_MAIN_BOUNDS k_bpr_main_tma(MainArgs a, Opt opt, int S) {
+__global__ void __launch_bounds__(256) k_bpr_main_tma(MainArgs a, Opt opt, int S) {
     extern __shared__ __align__(128) unsigned char dsm[];
     const unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -559,21 +552,14 @@ __global__ void DAISY_MAIN_BOUNDS k_bpr_main_tma(MainArgs a, Opt opt, int S) {
 template <int V>
 __device__ __forceinline__ void sum_staged(const float *__restrict__ stage, size_t q0, int len, int D4, int lane,
                                            const bool (&act)[V], float4 (&acc)[V]) {
-#ifdef DAISY_SEG_UN  // tools/small_book_probe.cu experiments
-    constexpr int UN = DAISY_SEG_UN;
-#else
     constexpr int UN = (V == 1) ? 8 : (V == 2 ? 4 : 2);
-#endif
-#ifndef DAISY_SEG_LD
-#define DAISY_SEG_LD ld_stream
-#endif
     for (int c = 0; c < len; c += UN) {
         float4 r[UN][V];
 #pragma unroll
         for (int jj = 0; jj < UN; ++jj)
 #pragma unroll
             for (int v = 0; v < V; ++v)
-                r[jj][v] = (c + jj < len && act[v]) ? DAISY_SEG_LD(stage, (q0 + c + jj) * D4 + lane + 32 * v) : f4_zero();
+                r[jj][v] = (c + jj < len && act[v]) ? ld_stream(stage, (q0 + c + jj) * D4 + lane + 32 * v) : f4_zero();
 #pragma unroll
         for (int jj = 0; jj < UN; ++jj)  // fixed order: sorted position ascending
             if (c + jj < len) {
@@ -608,20 +594,6 @@ __device__ __forceinline__ void seg_window(long long w, int tbl, const float *__
     bool act[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) act[v] = (lane + 32 * v) < D4;
-#ifdef DAISY_SEG_PREFETCH  // experiment knob: the warp walks its rows one after the other, each a DRAM round trip; ask L2 for the
-    // window's staged contributions (they sit at their sorted positions: one contiguous run) and table rows up front
-    {
-        const bool in_multi = valid && (prev == key || (next == key && p + 1 < n));
-        if (in_multi) {
-            const char *sp = reinterpret_cast<const char *>(stage + (size_t)p * D4 * 4);
-            for (int o = 0; o < D4 * 16; o += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(sp + o));
-        }
-        if (multi && (tbl == 0 || Opt::kNeedOldItem)) {
-            const char *tp = reinterpret_cast<const char *>(table + (size_t)key * D4 * 4);
-            for (int o = 0; o < D4 * 16; o += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(tp + o));
-        }
-    }
-#endif
 
     while (todo) {
         const int b = __ffs(todo) - 1;
@@ -674,13 +646,6 @@ __device__ __forceinline__ void seg_window(long long w, int tbl, const float *__
 // The accumulation order of a row is its sorted-ref order, fixed by the sort => bit-reproducible.  It differs from
 // the general path's order (which groups triples by positive item first), so the two paths agree to rounding only.
 // ------------------------------------------------------------------------------------------------
-#ifdef DAISY_SMALL_PROBE  // tools/small_book_probe.cu: clock stamps of thread 0 of each block
-__device__ long long g_small_probe[256][32];
-#define SMALL_PROBE(n) do { if (threadIdx.x == 0) g_small_probe[blockIdx.x][n] = clock64(); } while (0)
-#else
-#define SMALL_PROBE(n) do { } while (0)
-#endif
-
 // Block-wide stable LSD radix sort of up to 1024 * IPT 32-bit words on bits [lo, lo + nbits), digits of up to 9 bits
 // ranked the way CUB's onesweep ranks them: a warp counts its digits by matching lanes (lanes holding the same digit
 // find each other, the lowest one bumps the warp's histogram), one block scan over (digit, warp) turns the
@@ -704,7 +669,6 @@ __device__ __forceinline__ void block_sort_words(uint32_t (&keys)[IPT], int ipt,
         const uint32_t dmask = (uint32_t)NB - 1u;
         const int HS = NB + 1;  // row stride: (digit, warp) cells of one scan step fall into 32 different banks
         uint32_t *wh = hist + (size_t)w * HS;
-        SMALL_PROBE(2 + 6 * p);
         for (int i = lane; i < NB; i += 32) wh[i] = 0;
         __syncwarp();
         uint32_t rank[IPT];
@@ -731,9 +695,7 @@ __device__ __forceinline__ void block_sort_words(uint32_t (&keys)[IPT], int ipt,
                 __syncwarp();
             }
         }
-        SMALL_PROBE(3 + 6 * p);
         __syncthreads();
-        SMALL_PROBE(4 + 6 * p);
         // exclusive scan of the cells in (digit, warp) order: thread t owns E consecutive cells
         const int E = NB / 32;
         uint32_t sum = 0;
@@ -768,14 +730,11 @@ __device__ __forceinline__ void block_sort_words(uint32_t (&keys)[IPT], int ipt,
             *cell = run;
             run += c;
         }
-        SMALL_PROBE(5 + 6 * p);
         __syncthreads();
-        SMALL_PROBE(6 + 6 * p);
 #pragma unroll
         for (int k = 0; k < IPT; ++k)
             if (k < ipt) out[wh[(keys[k] >> shift) & dmask] + rank[k]] = keys[k];
         __syncthreads();
-        SMALL_PROBE(7 + 6 * p);
         if (p + 1 < passes) {
 #pragma unroll
             for (int k = 0; k < IPT; ++k)
@@ -820,7 +779,6 @@ __global__ void __launch_bounds__(1024) k_small_book(const int32_t *__restrict__
     const int vb = items ? vbQ : vbU, kb = items ? kbQ : kbU;
     const uint32_t bound = items ? I : U;
     uint32_t keys[IPT];
-    SMALL_PROBE(0);
     // ---- every ref of the table: mine / lower class / neither ----
     const bool checker = !items && cls == 0;  // this block also validates the triples and writes the clamped copy
 #pragma unroll
@@ -901,9 +859,7 @@ __global__ void __launch_bounds__(1024) k_small_book(const int32_t *__restrict__
         keys[k] = (k < ipt && q < n_c) ? sk[q] : 0xFFFFFFFFu;  // padding behind the real refs; the sort is stable
     }
     __syncthreads();
-    SMALL_PROBE(1);
     if (ipt > 0) block_sort_words<IPT>(keys, ipt, vb + DAISY_SMALL_CB, kb - DAISY_SMALL_CB, hist, sk, scan_tmp);
-    SMALL_PROBE(30);
     const uint32_t vmask = (1u << vb) - 1u;
     uint32_t *key_out = (items ? qkey_s : ukey_s) + base_c;
 #pragma unroll
@@ -944,7 +900,6 @@ __global__ void __launch_bounds__(1024) k_small_book(const int32_t *__restrict__
         else
             islot[idx - B] = slot;
     }
-    SMALL_PROBE(31);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -994,7 +949,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
     if (tid == 0) s_low = 0;
     for (int i = tid; i < 32 * 32 + 1; i += 1024) tw_off[i] = 0;
     __syncthreads();
-    SMALL_PROBE(0);
     // ---- sweep 1: how many refs of this class every (tile, warp) holds; how many refs belong to lower classes ----
     uint32_t low = 0;
     const bool checker = !items && cls == 0;  // this block also validates the triples and writes the clamped copy
@@ -1063,7 +1017,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
     for (int o = 16; o > 0; o >>= 1) low += __shfl_xor_sync(FULL, low, o);
     if (lane == 0 && low) atomicAdd(&s_low, low);
     __syncthreads();
-    SMALL_PROBE(1);
     // exclusive scan of the 1024 (tile, warp) counts: thread t owns cell t
     uint32_t n_c;
     {
@@ -1095,7 +1048,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
     __syncthreads();
     uint32_t *ak = ms.ak + tbl_off + base_c, *av = ms.av + tbl_off + base_c;
     uint32_t *bk = ms.bk + tbl_off + base_c, *bv = ms.bv + tbl_off + base_c;
-    SMALL_PROBE(2);
     // ---- sweep 2: compact this class's refs, in ref order, as (row >> cb, ref index) ----
     load_tile(0, nxt);
     for (int tl = 0; tl < tiles; ++tl) {
@@ -1117,7 +1069,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
         }
     }
     __syncthreads();  // (block-scope visibility of the global stores above)
-    SMALL_PROBE(3);
     // ---- LSD passes between (ak, av) and (bk, bv): warp w owns [w * len_w, (w + 1) * len_w) of the slice ----
     const uint32_t len_w = (((n_c + 31u) / 32u) + 31u) & ~31u;
     const uint32_t r0 = (uint32_t)w * len_w, r1 = min(r0 + len_w, n_c);
@@ -1214,7 +1165,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
         t = av; av = bv; bv = t;
         done += db;
     }
-    SMALL_PROBE(4);
     // ---- slots: (ak, av) is the class's slice, sorted by row, refs of a row in ref order ----
     uint32_t *key_out = (items ? qkey_s : ukey_s) + base_c;
     for (uint32_t p = tid; p < n_c; p += 1024) {
@@ -1249,7 +1199,6 @@ __global__ void __launch_bounds__(1024) k_mid_book(const int32_t *__restrict__ t
             }
         }
     }
-    SMALL_PROBE(5);
 }
 
 static int launch_mid_book(daisy_ctx *h, cudaStream_t bs, const int32_t *triples, int B, uint32_t U, uint32_t I, BookSet &k) {
@@ -1292,7 +1241,7 @@ static int launch_small_book(daisy_ctx *h, cudaStream_t bs, const int32_t *tripl
 // Every row with several contributions, both tables, ONE launch (all paths; in the row-sharded step `opt` is PushOpt,
 // which stores a finished item-row sum into its owner's memory over NVLink).
 //   blocks [0, NS)                  slice blocks: the rows the bookkeeping listed as longer than `long_len`.  One SM
-//        draws ~40 B/clk from L2 however many loads it has in flight (tools/small_book_probe.cu), so a hot row's
+//        draws ~40 B/clk from L2 however many loads it has in flight (DESIGN.md §4b), so a hot row's
 //        staged contributions are spread over the SMs slice by slice: a warp sums one slice of SLICE contributions
 //        into stage2, takes a ticket of its row, and the warp that draws the row's last ticket adds the slice sums
 //        IN SLICE ORDER and updates the row -- the order of the sum is fixed by the slice numbers, not by who
@@ -1301,16 +1250,8 @@ static int launch_small_book(daisy_ctx *h, cudaStream_t bs, const int32_t *tripl
 //        `long_len` contributions that start in its window
 //   the last block                  the loss reduction
 // ------------------------------------------------------------------------------------------------
-#if defined(DAISY_SEG_MIN_BLOCKS_V1)  // experiment knob: only the one-float4-per-lane instantiation (D <= 128, what config 4 runs;
-// 52 registers = 4 blocks per SM by default): 5 / 6 / 8 blocks per SM cap it at 48 / 40 / 32 registers (4 / 16 / 24 bytes spilled)
-#define DAISY_SEG_BOUNDS __launch_bounds__(256, (V == 1 ? DAISY_SEG_MIN_BLOCKS_V1 : 1))
-#elif defined(DAISY_SEG_MIN_BLOCKS)  // experiment knob (compile time): 2 caps k_seg_all at 128 registers -> two blocks per SM
-#define DAISY_SEG_BOUNDS __launch_bounds__(256, DAISY_SEG_MIN_BLOCKS)
-#else
-#define DAISY_SEG_BOUNDS __launch_bounds__(256)
-#endif
 template <int V, class Opt, int WIN, int SLICE>
-__global__ void DAISY_SEG_BOUNDS k_seg_all(const float *__restrict__ P, const float *__restrict__ Q,
+__global__ void __launch_bounds__(256) k_seg_all(const float *__restrict__ P, const float *__restrict__ Q,
                                                   const uint32_t *__restrict__ ukey_s,
                                                   const uint32_t *__restrict__ qkey_s, int B, int nQ, uint32_t q_sentinel,
                                                   const float *__restrict__ stageU, const float *__restrict__ stageQ,
@@ -1410,10 +1351,7 @@ __global__ void DAISY_SEG_BOUNDS k_seg_all(const float *__restrict__ P, const fl
 #pragma unroll
             for (int v = 0; v < V; ++v) grp[v] = f4_zero();
             const int g1 = min(nsl, g0 + 64);
-#ifndef DAISY_SEG_COMBINE_TILE  // slice sums in flight per warp of the combine tail (any value: same order of additions)
-#define DAISY_SEG_COMBINE_TILE 8
-#endif
-            constexpr int CT = DAISY_SEG_COMBINE_TILE;
+            constexpr int CT = 8;
             for (int j0 = g0; j0 < g1; j0 += CT) {
                 float4 rr[CT][V];
 #pragma unroll
@@ -1881,11 +1819,7 @@ static int table_phase_v(daisy_ctx *h, const StepPlan &pl, const float *P, const
     if ((size_t)S * stage_bytes > (size_t)56 * 1024) S = (int)((size_t)56 * 1024 / stage_bytes);
     if (pl.small) S = 0;  // one triple per warp: nothing to pipeline
     if (S >= 2) {
-        size_t smem = S * stage_bytes + (size_t)8 * S * 8;
-        if (h->main_max_blocks > 0) {  // experiment: leave room on every SM for the bookkeeping stream's blocks
-            const size_t floor_b = ((size_t)233472 / (size_t)(h->main_max_blocks + 1) + 1023) / 1024 * 1024;
-            if (floor_b > smem && floor_b <= (size_t)227 * 1024) smem = floor_b;
-        }
+        const size_t smem = S * stage_bytes + (size_t)8 * S * 8;
         static size_t granted_tab[2][64];  // per instantiation (V, Opt): shared memory already granted, by PTR and device
         size_t &granted = granted_tab[pl.jsrc ? 1 : 0][h->device & 63];
         if (pl.jsrc) {
@@ -1919,22 +1853,16 @@ static int table_phase_v(daisy_ctx *h, const StepPlan &pl, const float *P, const
                 P, Q, k.ukey_s, k.qkey_s, B, 2 * B, 0xFFFFFFFFu, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
                 DAISY_SMALL_SLICE, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, 0, nullptr);
         } else {
-            const int win = h->seg_win == 16 ? 16 : 32;  // DAISY_SEG_WIN: sorted refs per warp of the window blocks
-            blocksU = daisy_ceil_div(B, 8 * win), blocksQ = daisy_ceil_div(2 * (int64_t)B, 8 * win);
+            blocksU = daisy_ceil_div(B, 8 * 32), blocksQ = daisy_ceil_div(2 * (int64_t)B, 8 * 32);
             if (ilvQ) blocksQ = daisy_ceil_div(blocksQ, ilvQ) * ilvQ;
             if (pl.counts) {  // the merged sort holds only the refs of repeated rows, a count known on the device only
                 const int cap = DAISY_SEG_WIN_BLOCKS * h->num_sms;
                 if (blocksU > cap) blocksU = cap;
                 if (blocksQ > cap) blocksQ = cap;
             }
-            if (win == 16)
-                k_seg_all<V, Opt, 16, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
-                    P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-                    h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ, pl.counts);
-            else
-                k_seg_all<V, Opt, 32, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
-                    P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
-                    h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ, pl.counts);
+            k_seg_all<V, Opt, 32, DAISY_SLICE><<<NS + blocksU + blocksQ + (loss_accum ? 1 : 0), 256, 0, s>>>(
+                P, Q, k.ukey_s, k.qkey_s, B, 2 * B, pl.I, h->stageU, h->stageQ, h->stage2, D4, opt, NS, blocksU, blocksQ,
+                h->heavy_len, k.longs, h->longs_cap, h->ticket, h->loss_part, warps, loss_accum, ilvQ, pl.counts);
         }
         DAISY_LAUNCH_CHECK(h);
         for (int ph = PH_SEG_U; ph <= PH_LOSS; ++ph) phase_mark(h, ph, s);
@@ -1968,24 +1896,9 @@ static int run_step(daisy_ctx *h, const float *P, const float *Q, const int32_t 
     // local item shard
     const uint32_t U = (uint32_t)h->U, I = (uint32_t)(h->item_rows_override ? h->item_rows_override : h->I);
     StepPlan pl;
-    // SM partitioning (partition.cu): the table kernels run on the partition that excludes the bookkeeping stream's SMs,
-    // ordered after the caller's earlier work and before its later work by two events
-    const bool part = h->part_ok && h->pipeline && h->timing != 2;
-    cudaStream_t ks = s;
-    if (part) {
-        DAISY_CUDA(cudaEventRecord(h->part_ev_in, s));
-        DAISY_CUDA(cudaStreamWaitEvent(h->part_main_stream, h->part_ev_in, 0));
-        ks = h->part_main_stream;
-    }
-    int rc = book_phase(h, pl, triples, B, U, I, ks, host_src, inputs_ready, nullptr);
+    const int rc = book_phase(h, pl, triples, B, U, I, s, host_src, inputs_ready, nullptr);
     if (rc) return rc;
-    rc = table_phase<Opt>(h, pl, P, Q, opt, c2, loss_accum);
-    if (rc) return rc;
-    if (part) {
-        DAISY_CUDA(cudaEventRecord(h->part_ev_out, ks));
-        DAISY_CUDA(cudaStreamWaitEvent(s, h->part_ev_out, 0));
-    }
-    return DAISY_OK;
+    return table_phase<Opt>(h, pl, P, Q, opt, c2, loss_accum);
 }
 
 static int check_step_args(daisy_ctx *h, const void *P, const void *Q, const void *triples, int64_t B) {

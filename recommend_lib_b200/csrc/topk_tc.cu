@@ -47,11 +47,8 @@ constexpr int TN = 128;      // items per tile (UMMA N)
 constexpr int KATOM = 64;    // bf16 elements per 128-byte swizzle row
 constexpr int STAGES = 3;
 constexpr int ATOM_BYTES = 128 * 128;  // 128 rows x 128 bytes: one TMA box, 16 KB
-#ifndef DAISY_TC_EPI_WARPS
-#define DAISY_TC_EPI_WARPS 16
-#endif
-constexpr int EPI_WARPS = DAISY_TC_EPI_WARPS;  // epilogue warps (4, 8 or 16): EPI_WARPS / 4 per TMEM lane quarter, each takes an
-                                               // equal share of a tile's columns
+constexpr int EPI_WARPS = 16;  // epilogue warps: EPI_WARPS / 4 per TMEM lane quarter, each takes an equal share of a
+                               // tile's columns
 constexpr int TC_THREADS = 32 * (4 + EPI_WARPS);
 
 // ---- PTX wrappers ---------------------------------------------------------------------------------------------------
@@ -153,8 +150,6 @@ struct FilterArgs {
     int n_units;                // n_groups * n_chunks
     long long I;
     int *err;                   // handle error word: bit 256 = tensor-core pipeline timeout
-    int dbg_mode;               // DAISY_TC_DEBUG (timing experiments only, results are WRONG): 1 = the epilogue only reads TMEM,
-                                // 2 = it does not even read it
     unsigned long long *stats;  // optional (DAISY_TC_STATS=1): cycles the roles spent waiting, summed over CTAs -- [0] producer on
                                 // empty stages, [1] producer on A, [2] MMA on full stages, [3] MMA on drained accumulators,
                                 // [4] epilogue on complete accumulators, [5] epilogue busy, [6] kernel cycles (CTA 0)
@@ -321,12 +316,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_filter_tc(const __grid_consta
                     for (int cc = 0; cc < CHUNKS; ++cc) {
                         const int c = half * CHUNKS + cc;
                         float v[32];
-                        if (a.dbg_mode == 2) continue;
                         tc_ld32(tbase + (uint32_t)(c * 32), v);
-                        if (a.dbg_mode == 1) {
-                            if (v[0] == 1.2345e30f && v[31] == 1.2345e30f) a.cnt[row[mt]] = 0;  // keeps the load alive
-                            continue;
-                        }
                         // One warp per scheduler hides no latency, so the scan is written as independent operations: a
                         // max tree (4 sub-maxima of 8 scores, then their maximum) instead of 32 compares chained through
                         // one predicate; only a sub-group whose maximum reaches the threshold is looked at score by score.
@@ -603,7 +593,6 @@ int daisy_tc_filter(daisy_ctx *h, const float *P, const float *Q, const TcItems 
         a.I = h->I;
         a.err = h->err;
         a.stats = nullptr;
-        a.dbg_mode = getenv("DAISY_TC_DEBUG") ? atoi(getenv("DAISY_TC_DEBUG")) : 0;
         const char *st_env = getenv("DAISY_TC_STATS");
         unsigned long long *stats_dev = nullptr;
         if (st_env && atoi(st_env) > 0 && daisy_scratch_alloc(h, (void **)&stats_dev, (8 + 1024) * sizeof(unsigned long long), s) == cudaSuccess) {
@@ -654,7 +643,7 @@ int daisy_tc_filter(daisy_ctx *h, const float *P, const float *Q, const TcItems 
                     mx = hs[8 + b] > mx ? hs[8 + b] : mx;
                     sum += (double)hs[8 + b];
                 }
-                fprintf(stderr, "[k_filter_tc] CTA cycles min %llu mean %.0f max %llu (debug mode %d)\n", mn, sum / n, mx, a.dbg_mode);
+                fprintf(stderr, "[k_filter_tc] CTA cycles min %llu mean %.0f max %llu\n", mn, sum / n, mx);
                 fprintf(stderr, "[k_filter_tc] kernel %.0f cycles; per CTA, fraction of it: producer waits for a free stage %.3f, for A %.3f | "
                                 "MMA waits for a full stage %.3f, for a drained accumulator %.3f | epilogue (warp 4) waits for an accumulator "
                                 "%.3f, busy %.3f | units %d, tiles per chunk %d, reserve %d/%d\n",

@@ -27,7 +27,7 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 # switches this file sets; the cached default runs are made without them
-SWITCHES = ("DAISY_PIPELINE", "DAISY_COPY_STREAM", "DAISY_SEG_WIN", "DAISY_MERGED_SORT")
+SWITCHES = ("DAISY_PIPELINE", "DAISY_COPY_STREAM", "DAISY_MERGED_SORT")
 # ~50 ms of the caller's stream at B200 clocks: long enough that unordered bookkeeping would read a stale buffer
 SLEEP_CYCLES = 100_000_000
 
@@ -231,18 +231,6 @@ def test_host_copy_on_the_bookkeeping_stream_is_bit_identical(dev, monkeypatch, 
     (P0, Q0, batches), sync, ref = baseline(name)
     monkeypatch.setenv("DAISY_COPY_STREAM", "0")
     got = run("host", P0, Q0, batches, lr_for(len(batches[0])), WD, dev)
-    assert_oracle(got, ref, name)
-    assert_bit_identical(got, sync, name)
-
-
-@pytest.mark.parametrize("name", ["graphed", "direct"])
-def test_seg_window_16(dev, monkeypatch, name):
-    """DAISY_SEG_WIN=16 (k_seg_all<..., 16, ...>).  The window only decides which warp owns a row: a row is summed by
-    sum_staged from its first sorted position in sorted order whatever the window, and rows longer than heavy_len go
-    to the slice blocks either way.  So the result is bit-identical to the default window of 32."""
-    (P0, Q0, batches), sync, ref = baseline(name)
-    monkeypatch.setenv("DAISY_SEG_WIN", "16")
-    got = run("ready", P0, Q0, batches, lr_for(len(batches[0])), WD, dev)
     assert_oracle(got, ref, name)
     assert_bit_identical(got, sync, name)
 
