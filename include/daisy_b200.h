@@ -265,6 +265,14 @@ DAISY_API int daisy_topk_candidates(daisy_handle_t h, const float *P, const floa
 DAISY_API int daisy_topk_full(daisy_handle_t h, const float *P, const float *Q, const int32_t *users, int64_t N, int K,
                     const int64_t *excl_ptr, const int32_t *excl_idx, int32_t *out_item, float *out_score,
                     daisy_stream_t stream);
+/* Which strategy served the last daisy_topk_full call on h: *path = DAISY_TOPK_PATH_EXACT (materialised scores +
+ * radix select), _SIMT (fp32 CUDA-core candidate filter) or _TC (BF16 tensor-core candidate filter); *filtered = users
+ * whose top K came from the candidate list, *redone = users the exact path redid because their list overflowed or
+ * held fewer than K admissible items (both 0 on the exact path).  Host state only: no device call. */
+#define DAISY_TOPK_PATH_EXACT 0
+#define DAISY_TOPK_PATH_SIMT 1
+#define DAISY_TOPK_PATH_TC 2
+DAISY_API int daisy_topk_full_path(daisy_handle_t h, int *path, int64_t *filtered, int64_t *redone);
 
 /* ---- device-side negative sampler (SURVEY.md section 8f, row N1) ------------------------------------
  * Replaces BPRData.ng_sample (util/data_loader.py:680-690) + the DataLoader(shuffle=True) permutation

@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(_HERE, "libdaisy_b200" + ("_" + _VARIANT if _VARIANT els
 
 OK, EINVAL, ECUDA, EINDEX, EUNSUPPORTED, ENOMEM = 0, -1, -2, -3, -4, -5
 FLAG_EAGER_DECAY = 1
+TOPK_PATHS = ("exact", "filter-simt", "filter-tc")   # DAISY_TOPK_PATH_EXACT, _SIMT, _TC
 NUM_PHASES = 11
 PHASES = ("prep", "sort_i", "refs", "sort_u", "sort_q", "slots", "main", "seg_u", "seg_q", "heavy", "loss")
 
@@ -106,6 +107,7 @@ SIGNATURES = {
                             c_i64, c_vp, c_vp],
     "daisy_topk_candidates": [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp],
     "daisy_topk_full": [c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp],
+    "daisy_topk_full_path": [c_vp, ctypes.POINTER(c_i32), ctypes.POINTER(c_i64), ctypes.POINTER(c_i64)],
     "daisy_sample_triples": [c_vp, c_vp, c_i64, c_i32, c_vp, c_i64, ctypes.c_uint64, ctypes.c_uint32, c_i32, c_vp, c_vp],
     "daisy_route_triples": [c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp],
     "daisy_mf_fit": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, ctypes.POINTER(MFParams),
@@ -281,6 +283,13 @@ class Handle:
         f, r, cnt = c_f64(), c_f64(), c_i64()
         check(self.L.daisy_topk_tc_ms(self.ptr, ctypes.byref(f), ctypes.byref(r), ctypes.byref(cnt)))
         return f.value, r.value, cnt.value
+
+    def topk_full_path(self):
+        """(path, filtered, redone) of the last daisy_topk_full call: path is one of TOPK_PATHS, filtered the users
+        whose top K came from a candidate list, redone the users the exact path redid."""
+        path, filtered, redone = c_i32(), c_i64(), c_i64()
+        check(self.L.daisy_topk_full_path(self.ptr, ctypes.byref(path), ctypes.byref(filtered), ctypes.byref(redone)))
+        return TOPK_PATHS[path.value], filtered.value, redone.value
 
     def phase_ms(self):
         arr = (c_f64 * NUM_PHASES)()

@@ -173,6 +173,10 @@ struct daisy_ctx {
     // full-catalogue top-K workspace (grown on demand by daisy_topk_full)
     float *scores;          // [tile_users, item_num] score tile
     size_t scores_cap;      // floats
+    // what the last daisy_topk_full call did (daisy_topk_full_path): DAISY_TOPK_PATH_*, users whose top K the filter
+    // produced, users the exact fallback redid
+    int topk_path;
+    int64_t topk_filtered, topk_redone;
 
     // tuning (env overridable, see api.cu)
     int chunk;       // max positive-item run length handled by one warp in the main kernel (0 = auto)

@@ -303,15 +303,27 @@ __global__ void k_thr_from_topk(const float *__restrict__ top_scores, int r, int
 }
 
 // Exact top-K of one user's candidate list: bitonic sort of the 64-bit (score desc, item asc) keys in shared memory.
-// Excluded items (the user's training positives, CSR) are dropped first.  A user whose list overflowed, or holds
-// fewer than K admissible candidates, is handed to the exact fallback (flag in redo[m]).
+// Excluded items (the user's training positives, CSR) are dropped first; an exclusion id outside [0, I) raises the
+// handle's error flag, as k_mask does on the exact path.  A user whose list overflowed, holds fewer than K admissible
+// candidates, or whose K-th admissible candidate scores below the threshold thr[m] is handed to the exact fallback (flag
+// in redo[m]).  The last case needs a candidate list that is a superset: the list holds every item at or above thr, but
+// only some of those below (the tensor-core filter's margin), so once the exclusions reach below thr the best items
+// left need not be in it.
 __global__ void __launch_bounds__(1024) k_select_cand(const unsigned long long *__restrict__ cand_key,
-                                                       const int *__restrict__ cnt, int cap, int K, int64_t first_user,
+                                                       const int *__restrict__ cnt, const float *__restrict__ thr, int cap,
+                                                       int K, int64_t first_user,
                                                        const int64_t *__restrict__ excl_ptr,
-                                                       const int32_t *__restrict__ excl_idx, int32_t *__restrict__ out_item,
-                                                       float *__restrict__ out_score, int *__restrict__ redo) {
+                                                       const int32_t *__restrict__ excl_idx, int64_t I,
+                                                       int32_t *__restrict__ out_item, float *__restrict__ out_score,
+                                                       int *__restrict__ redo, int *err) {
     extern __shared__ unsigned long long keys[];
     const int m = blockIdx.x, tid = threadIdx.x;
+    if (excl_ptr && excl_idx)
+        for (int64_t e = excl_ptr[first_user + m] + tid; e < excl_ptr[first_user + m + 1]; e += blockDim.x)
+            if ((int64_t)(uint32_t)excl_idx[e] >= I) {
+                atomicOr(&err[0], 1);
+                atomicMin(&err[1], (int)(first_user + m));
+            }
     const int n = cnt[m];
     if (n > cap || n < K) {
         if (tid == 0) redo[m] = 1;
@@ -346,7 +358,8 @@ __global__ void __launch_bounds__(1024) k_select_cand(const unsigned long long *
             }
             __syncthreads();
         }
-    if (keys[K - 1] == 0ull) {  // fewer than K admissible candidates after the exclusions
+    // fewer than K admissible candidates after the exclusions, or the K-th of them below the threshold
+    if (keys[K - 1] == 0ull || okey_inv((uint32_t)(keys[K - 1] >> 32)) < thr[m]) {
         if (tid == 0) redo[m] = 1;
         return;
     }
@@ -366,6 +379,8 @@ extern "C" int daisy_topk_full(daisy_handle_t h, const float *P, const float *Q,
     DAISY_REQUIRE(h->D % 4 == 0, DAISY_EUNSUPPORTED, "daisy_topk_full needs dim %% 4 == 0 (dim is %d)", h->D);
     DAISY_REQUIRE(K >= 1 && K <= 128 && (int64_t)K <= h->I, DAISY_EUNSUPPORTED, "top_k %d unsupported (1..min(128, item_num))", K);
     DAISY_REQUIRE(N >= 0 && N < (1LL << 31), DAISY_EINVAL, "bad user count");
+    h->topk_path = DAISY_TOPK_PATH_EXACT;
+    h->topk_filtered = h->topk_redone = 0;
     if (N == 0) return DAISY_OK;
     DAISY_REQUIRE(users && out_item && out_score, DAISY_EINVAL, "null argument");
     DAISY_REQUIRE((excl_ptr == nullptr) == (excl_idx == nullptr) || excl_ptr != nullptr, DAISY_EINVAL,
@@ -432,6 +447,7 @@ extern "C" int daisy_topk_full(daisy_handle_t h, const float *P, const float *Q,
     // re-scoring of the candidates) unless DAISY_TOPK_TC=0 or the shape is outside its range (dim > 128)
     const char *tc_env = getenv("DAISY_TOPK_TC");
     const bool use_tc = !(tc_env && atoi(tc_env) == 0) && daisy_tc_supported(h);
+    h->topk_path = use_tc ? DAISY_TOPK_PATH_TC : DAISY_TOPK_PATH_SIMT;
     const int64_t Tu_max = use_tc ? 16384 : 4096;
     const int64_t Tu = N < Tu_max ? N : Tu_max;
     TcItems tci = {nullptr, nullptr, 0};
@@ -474,8 +490,8 @@ extern "C" int daisy_topk_full(daisy_handle_t h, const float *P, const float *Q,
                 k_score_tile<true><<<gf, 256, 0, s>>>(P, Q, users + first, nu, (uint32_t)h->U, I, h->D, c2, nullptr, h->err, thr,
                                                       cnt, cand, cap);
             }
-            k_select_cand<<<nu, 1024, cap * sizeof(unsigned long long), s>>>(cand, cnt, cap, K, first, excl_ptr, excl_idx,
-                                                                             out_item, out_score, redo + first);
+            k_select_cand<<<nu, 1024, cap * sizeof(unsigned long long), s>>>(cand, cnt, thr, cap, K, first, excl_ptr, excl_idx, I,
+                                                                             out_item, out_score, redo + first, h->err);
             h->launches += 5;
         }
         if (!rc && cudaGetLastError() != cudaSuccess) {
@@ -494,8 +510,20 @@ extern "C" int daisy_topk_full(daisy_handle_t h, const float *P, const float *Q,
         if (p) cudaFreeAsync(p, s);
     if (!rc)
         for (int64_t m = 0; m < N && !rc; ++m)
-            if (redo_host[m]) rc = exact_range(users + m, 1, m);
+            if (redo_host[m]) {
+                rc = exact_range(users + m, 1, m);
+                h->topk_redone++;
+            }
+    if (!rc) h->topk_filtered = N - h->topk_redone;
     free(redo_host);
     return rc;
+}
+
+extern "C" int daisy_topk_full_path(daisy_handle_t h, int *path, int64_t *filtered, int64_t *redone) {
+    DAISY_REQUIRE(h && path && filtered && redone, DAISY_EINVAL, "null argument");
+    *path = h->topk_path;
+    *filtered = h->topk_filtered;
+    *redone = h->topk_redone;
+    return DAISY_OK;
 }
 

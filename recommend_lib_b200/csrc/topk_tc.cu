@@ -7,14 +7,21 @@
 //
 // What the tensor cores compute is NOT the ranking score.  The exact path ranks by fp32 scores (fp32 products summed in
 // ascending k by fused multiply-adds); that arithmetic stays.  The tensor cores only answer "which items CAN be at or
-// above user u's threshold thr_u": with p~, q~ the BF16 roundings of the rows (|x~ - x| <= 2^-9 |x|),
-//     | sum_k p~_k q~_k  -  sum_k p_k q_k |  <=  (2^-8 + 2^-18) sum_k |p_k q_k|  <=  2^-8 (1 + 2^-10) |p_u| |q_i|
-// (BF16 x BF16 products are exact in fp32; the fp32 accumulation of <= 128 terms inside the tensor core and the
-// rounding of the exact path's own fma chain are covered by the slack kappa = 2^-8 * 17/16).  So every item whose
-// EXACT score reaches thr_u satisfies
-//     s~(u, i)  >=  thr_u / c^2  -  kappa |p_u| max_i |q_i|  =:  tau_u ,
-// and the epilogue appends exactly the items with s~ >= tau_u to the user's candidate list: a guaranteed superset
-// (about 15 % more candidates than the exact filter at the 10^-3 quantile).  k_rescore then recomputes the candidates'
+// above user u's threshold thr_u".  BF16 keeps 8 significant bits, so round-to-nearest gives p~, q~ with
+// |x~ - x| <= 2^-8 |x| (1 + 2^-8 rounds to 1), and per product |p~q~ - pq| <= (2 * 2^-8 + 2^-16) |pq|:
+//     | sum_k p~_k q~_k  -  sum_k p_k q_k |  <=  (2^-7 + 2^-16) sum_k |p_k q_k|  <=  2^-7 (1 + 2^-9) |p_u| |q_i|
+// (Cauchy-Schwarz for the last step).  BF16 x BF16 products are exact in fp32.  Two fp32 sums remain: the tensor
+// core's accumulation of D <= 128 terms and the exact path's fma chain over the same terms, each off by at most
+// gamma_D (1 + 2^-6) |p_u| |q_i| with gamma_D = D 2^-24 / (1 - D 2^-24) <= 2^-17 = 2^-7 * 2^-10 (twice that if the
+// tensor core truncates instead of rounding).  Together with the product term that is at most 2^-7 * 3 * 2^-9
+// |p_u| |q_i|, and kappa = 2^-7 * 17/16 leaves 2^-7 * 2^-4, more than ten times as much (the norms' own fp32 error is
+// covered by the 1.0001 by which k_rows_bf16 rounds them up).  So every item
+// whose EXACT score reaches thr_u satisfies
+//     s~(u, i)  >=  thr_u / c^2  -  kappa |p_u| max_{j in tile(i)} |q_j|  =:  tau_u,t ,
+// where tile(i) is the 128-item tile of i (the bound holds with |q_i| itself; the largest norm of the tile keeps it to
+// one fma per row and tile in the epilogue, and is far tighter than the catalogue-wide largest norm when row norms
+// spread: with log-normal norms of sigma 1 that one lets through ten times the candidates and overflows the list).
+// The epilogue appends exactly the items with s~ >= tau_u,t to the user's candidate list: a guaranteed superset.  k_rescore then recomputes the candidates'
 // scores with the exact path's arithmetic and k_select_cand (topk_full.cu) orders them, so the result is bit-identical
 // to the exact path -- tests/test_bpr_gpu.py::test_topk_full_*.
 //
@@ -140,6 +147,8 @@ constexpr uint32_t kIdesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TN 
 
 struct FilterArgs {
     const float *tau;           // [rows padded to 256] per-user threshold in accumulator units (+inf on padding rows)
+    const float *kp;            // [rows padded to 256] kappa |p_u|: the tile's threshold is tau - kp * tile_norm[t]
+    const float *tile_norm;     // [n_tiles] largest |q_i| of each item tile (rounded up)
     int *cnt;                   // [rows] candidates appended so far
     unsigned long long *cand;   // [rows, cap] candidate slots (low word = item id; k_rescore completes the key)
     int cap;
@@ -284,7 +293,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_filter_tc(const __grid_consta
             const int t0 = chunk * a.tiles_per_chunk;
             const int t1 = min(t0 + a.tiles_per_chunk, a.n_tiles);
             int row[MT];
-            float tau[MT];
+            float tau[MT], kp[MT];
             // Candidate slots are RESERVED in blocks: an atomicAdd that returns a position costs a global round trip
             // (~1 us) and the append cannot proceed without it.  A thread owns its (row, column half) for the whole
             // unit, so it takes reserve0 slots per row up front (the round trips of all rows overlap, nothing waits
@@ -295,6 +304,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_filter_tc(const __grid_consta
             for (int mt = 0; mt < MT; ++mt) {
                 row[mt] = g * (MT * TM) + mt * TM + q * 32 + lane;
                 tau[mt] = a.tau[row[mt]];
+                kp[mt] = a.kp[row[mt]];
                 nxt[mt] = end[mt] = 0;
                 if (tau[mt] < INFINITY) {
                     nxt[mt] = (uint32_t)atomicAdd(&a.cnt[row[mt]], a.reserve0);
@@ -307,11 +317,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_filter_tc(const __grid_consta
                 if (!ok) break;
                 tc_fence_after();
                 const long long i0 = (long long)t * TN;
+                const float qmax = __ldg(a.tile_norm + t);
 #pragma unroll
                 for (int mt = 0; mt < MT; ++mt) {
                     const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + ab * (uint32_t)(MT * TN) + (uint32_t)(mt * TN);
                     unsigned long long *slots = a.cand + (size_t)row[mt] * a.cap;
-                    const float th = tau[mt];
+                    const float th = fmaf(-kp[mt], qmax, tau[mt]);
 #pragma unroll 1
                     for (int cc = 0; cc < CHUNKS; ++cc) {
                         const int c = half * CHUNKS + cc;
@@ -371,12 +382,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_filter_tc(const __grid_consta
 }
 
 // ---- operand preparation --------------------------------------------------------------------------------------------
-// One warp per row: BF16 copy padded to Dp columns, Euclidean norm of the fp32 row.  users != nullptr gathers rows
+// One warp per row: BF16 copy padded to Dp columns, Euclidean norm of the fp32 row (into norm[w] and / or as the
+// maximum over the row's item tile, tile_norm_bits[w / TN]).  users != nullptr gathers rows
 // users[m] (validated: a bad id raises the handle's error flag and reads row 0); rows >= n_rows are zero padding.
 __global__ void __launch_bounds__(256) k_rows_bf16(const float *__restrict__ W, const int32_t *__restrict__ users,
                                                     long long n_rows, long long n_rows_padded, uint32_t limit, int D, int Dp,
                                                     __nv_bfloat16 *__restrict__ out, float *__restrict__ norm,
-                                                    unsigned *__restrict__ max_norm_bits, int *err) {
+                                                    unsigned *__restrict__ tile_norm_bits, int *err) {
     const int lane = threadIdx.x & 31;
     const long long w = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
     if (w >= n_rows_padded) return;
@@ -409,23 +421,26 @@ __global__ void __launch_bounds__(256) k_rows_bf16(const float *__restrict__ W, 
     const float nrm = sqrtf(ss) * 1.0001f;  // rounded up a little: the norm is used as an upper bound
     if (lane == 0) {
         if (norm) norm[w] = nrm;
-        if (max_norm_bits) atomicMax(max_norm_bits, __float_as_uint(nrm));  // non-negative floats order like their bits
+        if (tile_norm_bits) atomicMax(tile_norm_bits + w / TN, __float_as_uint(nrm));  // non-negative floats order like their bits
     }
 }
 
-// tau_u = thr_u / c^2 (moved down by 2^-20 of its magnitude: the exact path's final multiply by c^2 rounds)
-//         - kappa |p_u| max_i |q_i|;   +inf on padding rows; candidate counters cleared
-__global__ void k_tau(const float *__restrict__ thr, const float *__restrict__ pnorm, const unsigned *__restrict__ max_norm_bits,
-                      float inv_c2, int n, int n_padded, float *__restrict__ tau, int *__restrict__ cnt) {
+// tau_u = thr_u / c^2 (moved down by 2^-20 of its magnitude: the exact path's final multiply by c^2 rounds) and
+// kp_u = kappa |p_u|: the epilogue's threshold for item tile t is tau_u - kp_u tile_norm[t].  +inf / 0 on padding rows;
+// candidate counters cleared
+__global__ void k_tau(const float *__restrict__ thr, const float *__restrict__ pnorm, float inv_c2, int n, int n_padded,
+                      float *__restrict__ tau, float *__restrict__ kp, int *__restrict__ cnt) {
     const int m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= n_padded) return;
     if (m >= n) {
         tau[m] = INFINITY;
+        kp[m] = 0.f;
         return;
     }
-    const float kappa = 0.00390625f * 1.0625f;
+    const float kappa = 0.0078125f * 1.0625f;  // 2^-7 * 17/16: see the bound at the top of this file
     const float t = thr[m] * inv_c2;
-    tau[m] = t - fabsf(t) * 9.5367431640625e-7f - kappa * pnorm[m] * __uint_as_float(*max_norm_bits);
+    tau[m] = t - fabsf(t) * 9.5367431640625e-7f;
+    kp[m] = kappa * pnorm[m];
     cnt[m] = 0;
 }
 
@@ -533,28 +548,29 @@ int daisy_tc_prepare_items(daisy_ctx *h, const float *Q, TcItems *ti, cudaStream
     const int Dp = h->D <= 64 ? 64 : 128;
     ti->Dp = Dp;
     ti->Qb = nullptr;
-    ti->max_norm = nullptr;
+    ti->tile_norm = nullptr;
+    const size_t norm_bytes = (size_t)((h->I + TN - 1) / TN) * sizeof(unsigned);
     cudaError_t e = daisy_scratch_alloc(h, (void **)&ti->Qb, (size_t)h->I * Dp * 2, s);
-    if (e == cudaSuccess) e = daisy_scratch_alloc(h, (void **)&ti->max_norm, 256, s);
+    if (e == cudaSuccess) e = daisy_scratch_alloc(h, (void **)&ti->tile_norm, norm_bytes, s);
     if (e != cudaSuccess) {
         (void)cudaGetLastError();
         daisy_tc_free_items(ti, s);
         daisy_set_error("top-K tensor-core workspace allocation failed (%zu bytes of bf16 item rows)", (size_t)h->I * Dp * 2);
         return DAISY_ENOMEM;
     }
-    cudaMemsetAsync(ti->max_norm, 0, 256, s);
+    cudaMemsetAsync(ti->tile_norm, 0, norm_bytes, s);
     const long long rows = h->I;
     k_rows_bf16<<<daisy_ceil_div(rows, 8), 256, 0, s>>>(Q, nullptr, rows, rows, 0u, h->D, Dp, (__nv_bfloat16 *)ti->Qb, nullptr,
-                                                       ti->max_norm, h->err);
+                                                       (unsigned *)ti->tile_norm, h->err);
     h->launches++;
     return DAISY_OK;
 }
 
 void daisy_tc_free_items(TcItems *ti, cudaStream_t s) {
     if (ti->Qb) cudaFreeAsync(ti->Qb, s);
-    if (ti->max_norm) cudaFreeAsync(ti->max_norm, s);
+    if (ti->tile_norm) cudaFreeAsync(ti->tile_norm, s);
     ti->Qb = nullptr;
-    ti->max_norm = nullptr;
+    ti->tile_norm = nullptr;
 }
 
 // Candidate lists of users[0 .. nu) against the whole catalogue; thr [nu] are the users' thresholds in SCORE units
@@ -567,7 +583,7 @@ int daisy_tc_filter(daisy_ctx *h, const float *P, const float *Q, const TcItems 
     float *pnorm = nullptr, *tau = nullptr;
     cudaError_t e = daisy_scratch_alloc(h, &Pb, (size_t)rows_p * Dp * 2, s);
     if (e == cudaSuccess) e = daisy_scratch_alloc(h, (void **)&pnorm, (size_t)rows_p * 4, s);
-    if (e == cudaSuccess) e = daisy_scratch_alloc(h, (void **)&tau, (size_t)rows_p * 4, s);
+    if (e == cudaSuccess) e = daisy_scratch_alloc(h, (void **)&tau, (size_t)rows_p * 2 * 4, s);  // tau, then kp
     int rc = DAISY_OK;
     if (e != cudaSuccess) {
         (void)cudaGetLastError();
@@ -582,9 +598,11 @@ int daisy_tc_filter(daisy_ctx *h, const float *P, const float *Q, const TcItems 
     if (!rc) {
         k_rows_bf16<<<daisy_ceil_div(rows_p, 8), 256, 0, s>>>(P, users, nu, rows_p, (uint32_t)h->U, h->D, Dp, (__nv_bfloat16 *)Pb,
                                                              pnorm, nullptr, h->err);
-        k_tau<<<daisy_ceil_div(rows_p, 256), 256, 0, s>>>(thr, pnorm, ti->max_norm, 1.0f / c2, nu, rows_p, tau, cnt);
+        k_tau<<<daisy_ceil_div(rows_p, 256), 256, 0, s>>>(thr, pnorm, 1.0f / c2, nu, rows_p, tau, tau + rows_p, cnt);
         FilterArgs a;
         a.tau = tau;
+        a.kp = tau + rows_p;
+        a.tile_norm = ti->tile_norm;
         a.cnt = cnt;
         a.cand = cand;
         a.cap = cap;
@@ -607,6 +625,11 @@ int daisy_tc_filter(daisy_ctx *h, const float *P, const float *Q, const TcItems 
         int n_chunks = (int)(q_bytes * live / (48.0 * 1024 * 1024)) + 1;
         const int for_balance = (4 * grid + a.n_groups - 1) / a.n_groups;
         if (n_chunks < for_balance) n_chunks = for_balance;
+        // ... but few enough that the slots a row reserves up front (n_chunks * (EPI_WARPS / 4) * reserve0, at most
+        // 1.5 expected + 4 (EPI_WARPS / 4) n_chunks) leave half of cap to the candidates: k_select_cand counts
+        // reservations, used or not, and sends a row past cap to the exact fallback
+        const int max_chunks = (int)((cap / 2 - 1.5 * expected) / (4 * (EPI_WARPS / 4)));
+        if (n_chunks > max_chunks) n_chunks = max_chunks > 1 ? max_chunks : 1;
         if (n_chunks > a.n_tiles) n_chunks = a.n_tiles;
         a.tiles_per_chunk = (a.n_tiles + n_chunks - 1) / n_chunks;
         n_chunks = (a.n_tiles + a.tiles_per_chunk - 1) / a.tiles_per_chunk;

@@ -2,9 +2,9 @@
 #pragma once
 #include "ctx.cuh"
 
-struct TcItems {      // per daisy_topk_full call: BF16 copy of the item table and the largest item-row norm
+struct TcItems {      // per daisy_topk_full call: BF16 copy of the item table and the largest item-row norm per tile
     void *Qb;         // [item_num, Dp] bf16, Dp = 64 or 128
-    unsigned *max_norm;  // bits of max_i |q_i| (rounded up)
+    float *tile_norm;    // [ceil(item_num / 128)] max |q_i| over each 128-item tile (rounded up)
     int Dp;
 };
 

@@ -558,12 +558,16 @@ def test_route_triples_emulated_is_the_rank_share_of_every_global_batch(world, n
     assert L.emu_err_flag(h) == 0
 
 
-@pytest.mark.parametrize("I,D,N,K,paths", [(300, 16, 5, 10, ("exact",)), (33000, 8, 3, 10, ("exact", "filter"))])
+@pytest.mark.parametrize("I,D,N,K,paths", [(300, 16, 5, 10, ("exact",)), (131072, 8, 3, 10, ("exact", "filter"))])
 def test_full_catalogue_topk_emulated(monkeypatch, I, D, N, K, paths):
     """csrc/topk_full.cu (row A9, GPU-verified): both selection strategies under the emulation; the filtered path must
-    return exactly what the materialise-and-select path returns."""
+    return exactly what the materialise-and-select path returns.  The filter case needs I >= 131 072: below that the
+    sample threshold's rank passes 128 and the call takes the exact path whatever it is asked for.  Under the emulation
+    the filter is the CUDA-core one (the tensor-core kernel is outside its reach)."""
     L = _load("topk_full")
     L.daisy_topk_full.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]
+    L.daisy_topk_full_path.argtypes = [c_vp, ctypes.POINTER(c_i32), ctypes.POINTER(c_i64), ctypes.POINTER(c_i64)]
+    served = c_i32(), c_i64(), c_i64()
     rng = np.random.default_rng(I + N)
     U = 20
     P = rng.standard_normal((U, D)).astype(np.float32)
@@ -583,6 +587,9 @@ def test_full_catalogue_topk_emulated(monkeypatch, I, D, N, K, paths):
         rc = L.daisy_topk_full(h, _p(P), _p(Q), _p(users), N, K, _p(ptr), _p(idx) if len(idx) else None, _p(items), _p(scores), None)
         assert rc == 0, L.emu_last_error()
         assert L.emu_err_flag(h) == 0
+        assert L.daisy_topk_full_path(h, *map(ctypes.byref, served)) == 0
+        want = (1, N, 0) if path == "filter" else (0, 0, 0)                          # DAISY_TOPK_PATH_SIMT / _EXACT
+        assert tuple(v.value for v in served) == want, path
         out[path] = (items, scores)
         for n in range(N):
             r = ref[n].copy()
@@ -597,6 +604,15 @@ def test_full_catalogue_topk_emulated(monkeypatch, I, D, N, K, paths):
             assert set(np.nonzero(r > kth + 1e-3)[0].tolist()) <= set(got.tolist()) and r[got].min() >= kth - 1e-3
     if len(paths) == 2:
         assert np.array_equal(out["exact"][0], out["filter"][0]) and np.array_equal(out["exact"][1], out["filter"][1])
+        # an exclusion id outside the catalogue raises the error flag on the filtered path too, not only in k_mask
+        bad = idx.copy() if len(idx) else np.zeros(1, np.int32)
+        bad[-1] = I
+        ptr_bad = ptr.copy()
+        ptr_bad[-1] = len(bad)
+        h = _dims_handle(L, U, I, D)
+        rc = L.daisy_topk_full(h, _p(P), _p(Q), _p(users), N, K, _p(ptr_bad), _p(bad), _p(items), _p(scores), None)
+        assert rc == 0 and L.emu_err_flag(h) != 0 and L.emu_err_pos(h) == N - 1
+        assert L.daisy_topk_full_path(h, *map(ctypes.byref, served)) == 0 and served[0].value == 1
 
 
 # ------------------------------------------------------------------------------------------------ the gated GPU tests themselves
