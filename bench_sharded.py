@@ -251,9 +251,7 @@ def bench_sharded(args, cfg, metric, unit):
                                        ("block rows, triples routed to the user's owner, item rows + row gradients "
                                         "exchanged by NCCL all-to-all"),
                            "exchange": args.exchange, "peer_mapping": args.mapping if peer else None,
-                           "main_schedule": (f"chunks dealt round-robin over "
-                                             f"{os.environ.get('DAISY_SHARD_INTERLEAVE') or world} owner ranges "
-                                             f"(DAISY_SHARD_INTERLEAVE; 0 = sorted order)") if peer else None,
+                           "main_schedule": f"chunks dealt round-robin over {world} owner ranges" if peer else None,
                            "l2": "inputs larger than L2", "lazy_decay_materialized_in_timed_region": False,
                            "parity_selfcheck": parity},
                 "clocks": clocks.summary() if clocks is not None else None,

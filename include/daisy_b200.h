@@ -184,7 +184,7 @@ DAISY_API int daisy_shard_apply(daisy_handle_t h, float lr, float wd, daisy_stre
 DAISY_API int daisy_shard_materialize(daisy_handle_t h, float *P_local, daisy_stream_t stream);
 /* The schedule of the fused step kernel (no device call): *chunk = the chunk of sorted triples that warp `warp` of a
  * launch over `nchunks` chunks takes when the chunks are dealt round-robin over `interleave` ranges of the
- * owner-grouped order (DAISY_SHARD_INTERLEAVE, default = world size; 0 / 1 = sorted order), -1 if the warp has none.
+ * owner-grouped order (the sharded step uses interleave = world size; 0 / 1 = sorted order), -1 if the warp has none.
  * Every chunk is taken by exactly one warp of the ceil(nchunks / interleave) * interleave launched. */
 DAISY_API int daisy_shard_schedule(int warp, int nchunks, int interleave, int *chunk);
 /* Reporting: owner_off_out [world+1] = first cache row of every owner in the most recent step of this rank, so

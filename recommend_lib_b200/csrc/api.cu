@@ -179,7 +179,7 @@ extern "C" int daisy_create(daisy_handle_t *out, int device, int64_t user_num, i
             cudaEventCreateWithFlags(&h->book[i].freed, cudaEventDisableTiming);
             cudaEventCreateWithFlags(&h->book[i].copied, cudaEventDisableTiming);
         }
-        if (B > 0 && env_int("DAISY_COPY_STREAM", 1)) cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
+        if (B > 0) cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
         if (cudaDeviceSynchronize() != cudaSuccess) {
             daisy_set_error("workspace initialisation failed: %s", cudaGetErrorString(cudaGetLastError()));
             rc = DAISY_ECUDA;

@@ -107,7 +107,7 @@ struct daisy_shard {
     int prepared_set; // ... into this bookkeeping set
     int64_t prepared_B;
     void *plan;       // StepPlan of the prepared step (step_kernels.cuh), owned by shard.cu
-    int ilv;          // chunk interleave of the main kernel = world (DAISY_SHARD_INTERLEAVE; 0 / 1 = sorted order)
+    int ilv;          // chunk interleave of the main kernel = world (MainArgs::ilv)
     // phase profile (daisy_set_timing(h, 2)): bookkeeping, fetch, compute+push, barrier, apply, barrier
     cudaEvent_t pev[7];
     double pms[6];
@@ -137,7 +137,7 @@ struct daisy_ctx {
     BookSet book[DAISY_NSETS];
     int book_idx;
     cudaStream_t side_stream;
-    cudaStream_t copy_stream;  // H2D of *_step_host triples (DAISY_COPY_STREAM=0: on the bookkeeping stream)
+    cudaStream_t copy_stream;  // H2D of *_step_host triples when pipelined (created when max_batch > 0)
     cudaEvent_t ev_call;
     int pipeline;           // 1: bookkeeping on the side stream (default), 0: everything on the caller's stream
     int inputs_ready;       // 1: device triples passed to daisy_bpr_step are complete at call time (no stream dependency)

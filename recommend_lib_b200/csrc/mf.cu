@@ -194,8 +194,10 @@ struct OwnArgs {
     daisy_mf_params prm;
     unsigned long long stall_ns;
     int batch;                     // DAISY_MF_BATCH (default 1): batched groups (k_mf_owner)
-    unsigned poll_ns;              // DAISY_MF_POLL_NS (default 20): back-off between two polls of a version
 };
+
+// back-off between two polls of a version in k_mf_owner (200 and 1 000 ns were measured no different, DESIGN.md section 6)
+constexpr unsigned MF_OWNER_POLL_NS = 20;
 
 __device__ __forceinline__ unsigned ld_relaxed_u32(const unsigned *p) {
     unsigned v;
@@ -457,7 +459,7 @@ __global__ void __launch_bounds__(128) k_mf_owner(OwnArgs a) {
                             unsigned spins = 0;
                             StallWatch watch;
                             while (ld_acquire_u32(&a.ver_u[u]) != want) {
-                                __nanosleep(a.poll_ns);
+                                __nanosleep(MF_OWNER_POLL_NS);
                                 if ((++spins & 0xfffu) == 0 && watch.stalled(a.progress, a.abort_flag, a.stall_ns)) {
                                     bail = 1;
                                     break;
@@ -533,7 +535,7 @@ __global__ void __launch_bounds__(128) k_mf_owner(OwnArgs a) {
                     unsigned spins = 0;
                     StallWatch watch;
                     while (ld_acquire_u32(&a.ver_u[u]) != want) {
-                        __nanosleep(a.poll_ns);
+                        __nanosleep(MF_OWNER_POLL_NS);
                         if ((++spins & 0xfffu) == 0 && watch.stalled(a.progress, a.abort_flag, a.stall_ns)) {
                             bail = 1;
                             break;
@@ -869,11 +871,7 @@ extern "C" int daisy_mf_fit(daisy_handle_t h, double *pu, double *qi, double *bu
         DAISY_CUDA(DVsel == 1 ? OCC_(1) : DVsel == 2 ? OCC_(2) : DVsel == 4 ? OCC_(4) : DVsel == 8 ? OCC_(8) : OCC_(16));
 #undef OCC_
         if (occ < 1) occ = 1;
-        int per_sm = occ < 8 ? occ : 8;
-        {
-            const char *env = getenv("DAISY_MF_BLOCKS_PER_SM");
-            if (env && atoi(env) > 0 && atoi(env) < per_sm) per_sm = atoi(env);
-        }
+        const int per_sm = occ < 8 ? occ : 8;
         const unsigned W = (unsigned)(h->num_sms * per_sm * 4);
         uint32_t *hkey, *hkey_s, *hval, *hval_s, *rank;
         int *lk_u, *lk_i;
@@ -916,12 +914,8 @@ extern "C" int daisy_mf_fit(daisy_handle_t h, double *pu, double *qi, double *bu
         o.wptr = wptr; o.ver_u = ver_u; o.err2 = err2; o.abort_flag = abort_flag;
         o.n = n; o.epochs = n_epochs; o.D = h->D; o.prm = *prm;
         o.stall_ns = stall_ns;
-        {
-            const char *be = getenv("DAISY_MF_BATCH");
-            o.batch = (be && *be) ? (atoi(be) != 0) : 1;
-            const char *pe = getenv("DAISY_MF_POLL_NS");
-            o.poll_ns = (pe && atoi(pe) > 0) ? (unsigned)atoi(pe) : 20u;
-        }
+        const char *be = getenv("DAISY_MF_BATCH");
+        o.batch = (be && *be) ? (atoi(be) != 0) : 1;
         o.progress = ticket;   // the ticket word is free under this schedule
         o.stats = nullptr;
         const char *st_env = getenv("DAISY_MF_STATS");
@@ -959,9 +953,7 @@ extern "C" int daisy_mf_fit(daisy_handle_t h, double *pu, double *qi, double *bu
         int occ = 0;
         DAISY_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_mf_dataflow, 128, 0));
         if (occ < 1) occ = 1;
-        int per_sm = occ < 8 ? occ : 8;
-        const char *env = getenv("DAISY_MF_BLOCKS_PER_SM");
-        if (env && atoi(env) > 0) per_sm = atoi(env) < occ ? atoi(env) : occ;
+        const int per_sm = occ < 8 ? occ : 8;
         k_mf_dataflow<<<h->num_sms * per_sm, 128, 0, s>>>(a);
         DAISY_LAUNCH_CHECK(h);
     }

@@ -801,11 +801,7 @@ extern "C" int daisy_shard_init(daisy_handle_t h, int rank, int world, int64_t i
     DAISY_REQUIRE(sh != nullptr, DAISY_ENOMEM, "host allocation failed");
     sh->rank = rank;
     shard_layout(sh, h->D, h->maxB, world, item_num_global);
-    {   // schedule of the main kernel: chunks dealt round-robin over `world` ranges of the owner-grouped order
-        const char *v = getenv("DAISY_SHARD_INTERLEAVE");
-        sh->ilv = (v && *v) ? atoi(v) : world;
-        if (sh->ilv < 0 || sh->ilv > 1024) sh->ilv = world;
-    }
+    sh->ilv = world;   // schedule of the main kernel: chunks dealt round-robin over `world` ranges of the owner-grouped order
     const size_t D = (size_t)h->D, cap = (size_t)sh->cap;
     h->sh = sh;
     bool ok = true;

@@ -1698,7 +1698,7 @@ static int book_phase(daisy_ctx *h, StepPlan &pl, const int32_t *triples, int64_
         // adds to the chain's 0.56 ms -- more than the 0.65 ms the table kernels take, so the COPY set the pace of the
         // host-fed step (0.75 ms against 0.70 from device-resident triples, profiles/r02g).  The copy of step n+2 now
         // runs under the bookkeeping of step n+1; the landing zone is the set's own (free once the set is).
-        if (piped && h->copy_stream) {
+        if (piped) {
             DAISY_CUDA(cudaStreamWaitEvent(h->copy_stream, k.freed, 0));
             DAISY_CUDA(cudaMemcpyAsync((void *)triples, host_src, (size_t)B * 3 * sizeof(int32_t), cudaMemcpyHostToDevice,
                                        h->copy_stream));

@@ -23,9 +23,6 @@
 //                      A history that holds an item m times (a repeated (user, item) rating) applies that row's update
 //                      m times in a row from the thread owning its first occurrence (`ur_mult`), which is what the
 //                      reference's `for j in Iu` does.
-//   k_svdpp_hot        picks the most frequent items of the histories; k_svdpp_seq keeps THEIR yj rows in the shared memory
-//                      the block does not otherwise need (~1 000 rows at n_factors 20) for the whole fit and writes them
-//                      back at the end, so most of a rating's gather / rewrite never leaves the SM (DAISY_SVDPP_HOT=0: off)
 //   k_svdpp_user_factors   z[u] = pu[u] + sum_{j in Iu} yj[j] / sqrt|Iu| (:281-286), a warp per user; predict is then
 //                      daisy_mf_predict(z, qi, bu, bi) -- the history is summed once per user, not once per candidate.
 //
@@ -57,9 +54,8 @@ struct SpArgs {
     const int32_t *ur_idx, *ur_mult;   // ur_mult may be null: no item repeats inside a list
     double *sse_out;                   // [epochs] or null
     const int *err;
-    const int *slot;                   // [I] shared-memory slot of item j's yj row, or -1 (null: no resident rows)
     long long n;
-    int epochs, D, H, I;               // H = resident rows
+    int epochs, D;
     daisy_svdpp_params prm;
 };
 
@@ -81,37 +77,6 @@ __global__ void k_svdpp_validate(const int32_t *users, const int32_t *items, lon
         if (ur_idx[k] < 0 || ur_idx[k] >= I) atomicOr(err, 2);
 }
 
-// The H most frequent items of the histories get a shared-memory slot for their yj row (k_svdpp_seq keeps those rows
-// on chip for the whole fit): count occurrences, bisect the smallest count threshold that selects at most H items,
-// hand out slots (which slot an item gets does not matter: the arithmetic is the same wherever the row lives).
-__global__ void __launch_bounds__(1024) k_svdpp_hot(const int64_t *ur_ptr, const int32_t *ur_idx, long long U, int I, int H,
-                                                    const int *err, int *cnt, int *slot) {
-    __shared__ int s_n;
-    const int tid = threadIdx.x, T = blockDim.x;
-    for (int j = tid; j < I; j += T) slot[j] = -1;
-    if (err[0] != 0) return;
-    const long long total = ur_ptr[U];
-    for (long long k = tid; k < total; k += T) atomicAdd(&cnt[ur_idx[k]], 1);
-    __syncthreads();
-    int lo = 1, hi = 0x40000000;
-    while (lo < hi) {                       // block-uniform: every thread reads the same s_n
-        const int mid = lo + (hi - lo) / 2;
-        if (tid == 0) s_n = 0;
-        __syncthreads();
-        int mine = 0;
-        for (int j = tid; j < I; j += T) mine += cnt[j] >= mid;
-        if (mine) atomicAdd(&s_n, mine);
-        __syncthreads();
-        const int n = s_n;
-        __syncthreads();
-        if (n <= H) hi = mid; else lo = mid + 1;
-    }
-    if (tid == 0) s_n = 0;
-    __syncthreads();
-    for (int j = tid; j < I; j += T)
-        if (cnt[j] >= lo) slot[j] = atomicAdd(&s_n, 1);
-}
-
 template <int M>
 __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) {   // D > 128: 512 threads, 128 registers
     extern __shared__ double sp_smem[];
@@ -125,7 +90,6 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
     SpHdr *hdr = reinterpret_cast<SpHdr *>(nb + 2);              // [3]     ring: current, next, the one being fetched
     int *list = reinterpret_cast<int *>(hdr + 3);                // [2][SP_CAP] item ids of the current / next history
     int *mlist = list + 2 * SP_CAP;                              // [2][SP_CAP] their multiplicities
-    double *hot = reinterpret_cast<double *>(mlist + 2 * SP_CAP);   // [H][D] resident yj rows (authoritative during the fit)
     if (a.err[0] != 0) return;              // an id failed validation: touch nothing (block-uniform)
     const long long total = a.n * (long long)a.epochs;
     if (total == 0) return;
@@ -141,27 +105,13 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
         h->p0 = p0;
         h->nI = (int)(a.ur_ptr[u + 1] - p0);
     };
-    auto enc = [&](int j) -> int {          // item id, or -1 - slot when its row is resident in shared memory
-        if (!a.slot) return j;
-        const int sl = a.slot[j];
-        return sl >= 0 ? -1 - sl : j;
-    };
     auto copy_list = [&](const SpHdr *h, int buf) {   // all threads
         const int m = h->nI < SP_CAP ? h->nI : SP_CAP;
         for (int k = tid; k < m; k += T) {
-            list[buf * SP_CAP + k] = enc(a.ur_idx[h->p0 + k]);
+            list[buf * SP_CAP + k] = a.ur_idx[h->p0 + k];
             mlist[buf * SP_CAP + k] = a.ur_mult ? a.ur_mult[h->p0 + k] : 1;
         }
     };
-    auto row_of = [&](int e) -> double * {  // a list entry -> its yj row, on chip or in global memory
-        return e < 0 ? hot + (size_t)(-1 - e) * D : a.yj + (size_t)e * D;
-    };
-    if (a.slot)                             // resident rows in
-        for (int j = w; j < a.I; j += W) {
-            const int sl = a.slot[j];
-            if (sl >= 0)
-                for (int f = lane; f < D; f += 32) hot[(size_t)sl * D + f] = a.yj[(size_t)j * D + f];
-        }
 
     // Everything a rating needs besides the history rows travels ahead of it, so that no dependent load sits between two
     // of its barriers: the header (u, i, r, list range) two ratings ahead -- ids fetched at the top of a rating, the list
@@ -222,7 +172,7 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
         for (int j = 0; j < KEEP; ++j) {
             const int k = w + j * W;
             const bool on = k < nI;         // warp-uniform
-            const double *row = on ? row_of(k < SP_CAP ? lst[k] : enc(a.ur_idx[p0 + k])) : nullptr;
+            const double *row = on ? a.yj + (size_t)(k < SP_CAP ? lst[k] : a.ur_idx[p0 + k]) * D : nullptr;
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const int f = lane + 32 * m;
@@ -235,7 +185,7 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
             for (int m = 0; m < M; ++m)
                 if (w + j * W < nI) acc[m] += keep[j][m];
         for (int k = w + KEEP * W; k < nI; k += W) {
-            const double *row = row_of(k < SP_CAP ? lst[k] : enc(a.ur_idx[p0 + k]));
+            const double *row = a.yj + (size_t)(k < SP_CAP ? lst[k] : a.ur_idx[p0 + k]) * D;
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const int f = lane + 32 * m;
@@ -313,7 +263,7 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
             if (k >= nI) break;             // warp-uniform
             const int mult = k < SP_CAP ? mls[k] : (a.ur_mult ? a.ur_mult[p0 + k] : 1);
             if (mult == 0) continue;        // a later occurrence of an item: its first occurrence applies both
-            double *row = row_of(k < SP_CAP ? lst[k] : enc(a.ur_idx[p0 + k]));
+            double *row = a.yj + (size_t)(k < SP_CAP ? lst[k] : a.ur_idx[p0 + k]) * D;
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const int f = lane + 32 * m;
@@ -327,7 +277,7 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
         for (int k = w + KEEP * W; k < nI; k += W) {
             const int mult = k < SP_CAP ? mls[k] : (a.ur_mult ? a.ur_mult[p0 + k] : 1);
             if (mult == 0) continue;        // a later occurrence of an item: its first occurrence applies both
-            double *row = row_of(k < SP_CAP ? lst[k] : enc(a.ur_idx[p0 + k]));
+            double *row = a.yj + (size_t)(k < SP_CAP ? lst[k] : a.ur_idx[p0 + k]) * D;
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const int f = lane + 32 * m;
@@ -355,12 +305,6 @@ __global__ void __launch_bounds__(M >= 8 ? 512 : 1024, 1) k_svdpp_seq(SpArgs a) 
         }
         if (++t2 == a.n) t2 = 0;
     }
-    if (a.slot)                             // resident rows out (the loop's last barrier ordered the final updates)
-        for (int j = w; j < a.I; j += W) {
-            const int sl = a.slot[j];
-            if (sl >= 0)
-                for (int f = lane; f < D; f += 32) a.yj[(size_t)j * D + f] = hot[(size_t)sl * D + f];
-        }
 }
 
 // z[u] = pu[u] + sum_{j in Iu} yj[j] / sqrt|Iu|   (SVDpp.predict, :281-286; a user without history keeps pu[u])
@@ -380,14 +324,13 @@ __global__ void k_svdpp_user_factors(const double *pu, const double *yj, const i
     }
 }
 
-static size_t sp_smem_bytes(int threads, int D, int H = 0) {
-    return (size_t)H * D * sizeof(double) + ((size_t)(threads / 32) * D + (size_t)D + 32 + 2) * sizeof(double) + 3 * sizeof(SpHdr) +
-           4 * (size_t)SP_CAP * sizeof(int);
+static size_t sp_smem_bytes(int threads, int D) {
+    return ((size_t)(threads / 32) * D + (size_t)D + 32 + 2) * sizeof(double) + 3 * sizeof(SpHdr) + 4 * (size_t)SP_CAP * sizeof(int);
 }
 
 template <int M>
 static int sp_launch(daisy_ctx *h, const SpArgs &a, int threads, cudaStream_t s) {
-    const size_t smem = sp_smem_bytes(threads, a.D, a.H);
+    const size_t smem = sp_smem_bytes(threads, a.D);
     DAISY_CUDA(cudaFuncSetAttribute(k_svdpp_seq<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_svdpp_seq<M><<<1, threads, smem, s>>>(a);
     DAISY_LAUNCH_CHECK(h);
@@ -432,36 +375,14 @@ extern "C" int daisy_svdpp_fit(daisy_handle_t h, double *pu, double *qi, double 
     a.n = (long long)n;
     a.epochs = n_epochs;
     a.D = D;
-    a.I = (int)h->I;
     a.prm = *prm;
-    // resident rows: what is left of the 227 KB of shared memory can hold the yj rows of the most frequent items.
-    // OFF by default since it was measured (profiles/r02a_bench_svdpp*.json, n_factors 20: 203 k ratings/s without,
-    // 189 k with: a 160-byte row comes from L2 as fast as the slot indirection costs); DAISY_SVDPP_HOT=<rows> enables it
-    // (results are bit-identical either way, tests/test_svdpp_gpu.py).
-    const size_t budget = 224 * 1024, base = sp_smem_bytes(threads, D);
-    long long H = base < budget ? (long long)((budget - base) / ((size_t)D * sizeof(double))) : 0;
-    if (const char *e = getenv("DAISY_SVDPP_HOT")) H = atoll(e) < H ? atoll(e) : H;
-    else H = 0;
-    if (H > h->I) H = h->I;
-    if (H < 0 || h->I > 0x7fffffffLL) H = 0;
-    a.H = (int)H;
-    a.slot = nullptr;
-    int *hotbuf = nullptr;
-    if (H > 0) {
-        DAISY_CUDA(daisy_scratch_alloc(h, (void **)&hotbuf, 2 * (size_t)h->I * sizeof(int), s));
-        DAISY_CUDA(cudaMemsetAsync(hotbuf, 0, 2 * (size_t)h->I * sizeof(int), s));
-        k_svdpp_hot<<<1, 1024, 0, s>>>(ur_ptr, ur_idx, (long long)h->U, (int)h->I, (int)H, h->err, hotbuf, hotbuf + h->I);
-        DAISY_LAUNCH_CHECK(h);
-        a.slot = hotbuf + h->I;
-    }
-    int rc;
-    if (D <= 32) rc = sp_launch<1>(h, a, threads, s);
-    else if (D <= 64) rc = sp_launch<2>(h, a, threads, s);
-    else if (D <= 128) rc = sp_launch<4>(h, a, threads, s);
-    else if (D <= 256) rc = sp_launch<8>(h, a, threads, s);
-    else rc = sp_launch<16>(h, a, threads, s);
-    if (hotbuf) cudaFreeAsync(hotbuf, s);
-    return rc;
+    // No yj rows are kept resident in shared memory: measured at n_factors 20, 203 k ratings/s without them and 189 k
+    // with (a row comes from L2 as fast as the slot indirection costs), so that option was removed (it is in git history).
+    if (D <= 32) return sp_launch<1>(h, a, threads, s);
+    if (D <= 64) return sp_launch<2>(h, a, threads, s);
+    if (D <= 128) return sp_launch<4>(h, a, threads, s);
+    if (D <= 256) return sp_launch<8>(h, a, threads, s);
+    return sp_launch<16>(h, a, threads, s);
 }
 
 extern "C" int daisy_svdpp_user_factors(daisy_handle_t h, const double *pu, const double *yj, const int64_t *ur_ptr,

@@ -27,7 +27,7 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 # switches this file sets; the cached default runs are made without them
-SWITCHES = ("DAISY_PIPELINE", "DAISY_COPY_STREAM", "DAISY_MERGED_SORT")
+SWITCHES = ("DAISY_PIPELINE", "DAISY_MERGED_SORT")
 # ~50 ms of the caller's stream at B200 clocks: long enough that unordered bookkeeping would read a stale buffer
 SLEEP_CYCLES = 100_000_000
 
@@ -221,16 +221,6 @@ def test_pipeline_off_is_bit_identical(dev, monkeypatch, name):
     (P0, Q0, batches), sync, ref = baseline(name)
     monkeypatch.setenv("DAISY_PIPELINE", "0")
     got = run("ready", P0, Q0, batches, lr_for(len(batches[0])), WD, dev)
-    assert_oracle(got, ref, name)
-    assert_bit_identical(got, sync, name)
-
-
-@pytest.mark.parametrize("name", list(SHAPES))
-def test_host_copy_on_the_bookkeeping_stream_is_bit_identical(dev, monkeypatch, name):
-    """DAISY_COPY_STREAM=0: the H2D copy of host triples runs on the bookkeeping stream instead of its own."""
-    (P0, Q0, batches), sync, ref = baseline(name)
-    monkeypatch.setenv("DAISY_COPY_STREAM", "0")
-    got = run("host", P0, Q0, batches, lr_for(len(batches[0])), WD, dev)
     assert_oracle(got, ref, name)
     assert_bit_identical(got, sync, name)
 

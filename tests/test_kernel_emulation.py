@@ -368,17 +368,15 @@ def test_svdpp_kernels_emulated_match_the_reference_golden_run(golden, monkeypat
     assert e.L.emu_err_flag(e.h) == 0
 
 
-@pytest.mark.parametrize("U,I,D,n,E,threads,hot", [(17, 23, 44, 260, 2, 64, 5),    # D > 32, ragged; 5 of 23 yj rows resident on chip
-                                                   (9, 12, 130, 90, 1, 160, 0),    # D > 128, 5 warps; no resident rows
-                                                   (1, 40, 8, 2100, 1, 64, None)]) # a history longer than the shared-memory list; all rows resident
-def test_svdpp_kernels_emulated_match_the_oracle_and_flag_bad_ids(monkeypatch, U, I, D, n, E, threads, hot):
+@pytest.mark.parametrize("U,I,D,n,E,threads", [(17, 23, 44, 260, 2, 64),     # D > 32, ragged
+                                              (9, 12, 130, 90, 1, 160),     # D > 128, 5 warps
+                                              (1, 40, 8, 2100, 1, 64)])     # a history longer than the shared-memory list
+def test_svdpp_kernels_emulated_match_the_oracle_and_flag_bad_ids(monkeypatch, U, I, D, n, E, threads):
     from oracle import mf_oracle
     monkeypatch.setenv("DAISY_SVDPP_THREADS", str(threads))
-    if hot is not None:
-        monkeypatch.setenv("DAISY_SVDPP_HOT", str(hot))
     rng = np.random.default_rng(U * 1000 + D)
     users = rng.integers(0, max(U - 2, 1), n)                       # the last users have no rating at all
-    items = (rng.zipf(1.3, n) - 1) % I                              # skewed, so that "the most frequent rows" is a real choice
+    items = (rng.zipf(1.3, n) - 1) % I                              # skewed: items repeat across and within histories
     users[5], items[5] = users[4], items[4]                         # a repeated (user, item) pair for sure
     ratings = rng.integers(1, 6, n).astype(np.float64)
     pu0, qi0, yj0 = (rng.normal(0, .1, s) for s in ((U, D), (I, D), (I, D)))

@@ -5,8 +5,6 @@ and the C oracle (oracle/mf_oracle.c: mf_oracle_svdpp_fit, bit-identical to that
 First run on a B200 in round 2 (profiles/r02a_*).
 float64 on both sides; two sums are re-associated on the device (history rows over warps, factors over lanes), so
 agreement is to rounding (1e-9 relative, as for funk-SVD), the sequential update ORDER is the reference's."""
-import os
-
 import numpy as np
 import pytest
 
@@ -88,17 +86,6 @@ def test_svdpp_against_c_oracle(U, I, D, n, E):
     assert np.isclose(a.sse_[E - 1], ref["sse"], rtol=1e-9)
     b = fit_from(SVDpp(U, I, n_factors=D, n_epochs=E, verbose=False), users, items, ratings, pu0, qi0, yj0)
     assert np.array_equal(a.yj, b.yj) and np.array_equal(a.pu, b.pu)      # run-to-run bit-reproducible
-    old = os.environ.get("DAISY_SVDPP_HOT")
-    os.environ["DAISY_SVDPP_HOT"] = "100000"                              # the most frequent yj rows resident in shared memory
-                                                                          # (as many as fit; off by default): same arithmetic
-    try:
-        c = fit_from(SVDpp(U, I, n_factors=D, n_epochs=E, verbose=False), users, items, ratings, pu0, qi0, yj0)
-    finally:
-        if old is None:
-            del os.environ["DAISY_SVDPP_HOT"]
-        else:
-            os.environ["DAISY_SVDPP_HOT"] = old
-    assert np.array_equal(a.yj, c.yj) and np.array_equal(a.qi, c.qi) and np.array_equal(a.bu, c.bu)
 
 
 def test_svdpp_bad_item_raises_and_leaves_no_partial_state():
