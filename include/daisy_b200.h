@@ -440,6 +440,23 @@ DAISY_API int daisy_neumf_forward(daisy_handle_t h, const daisy_neumf_params *p,
 DAISY_API int daisy_neumf_step(daisy_handle_t h, const daisy_neumf_params *p, const int32_t *samples, int64_t B,
                      int64_t step_no, void *scratch, int64_t scratch_bytes, double *loss_accum, daisy_stream_t stream);
 
+/* Ranking with the tower: score(u, i) = the logit NCF.forward returns (NCFRecommender.py:105-125), up to the fp32
+ * reassociation of layer 0, which is split into a per-user and a per-item half.  Only the forward fields of p are read
+ * (the Adam moment pointers may be NULL).  Scores are fp32 sums in a fixed order: a user's results are the same bits
+ * whether it is ranked alone or with others, and in both entry points.
+ * metric_eval(model, test_loader, top_k, algo='ncf') -> _ncf_topk (util/metrics.py:68-86,88-94), all groups at once:
+ * for n < N the K best of score(users[n], cand[n,c]), c < C, in (score desc, position asc) order; out_pos [N,K] =
+ * candidate positions, out_item [N,K] = cand ids, out_score [N,K].  C <= 8192, K <= 128, K <= C
+ * (the layout of daisy_topk_candidates). */
+DAISY_API int daisy_neumf_topk_candidates(daisy_handle_t h, const daisy_neumf_params *p, const int32_t *users,
+                                          const int32_t *cand, int64_t N, int C, int K, int32_t *out_pos,
+                                          int32_t *out_item, float *out_score, daisy_stream_t stream);
+/* Full catalogue: for n < N the K best items of score(users[n], i), i < item_num, order (score desc, item asc), with
+ * optional CSR exclusion lists (the user's training positives) as in daisy_topk_full.  K <= 128. */
+DAISY_API int daisy_neumf_topk_full(daisy_handle_t h, const daisy_neumf_params *p, const int32_t *users, int64_t N, int K,
+                                    const int64_t *excl_ptr, const int32_t *excl_idx, int32_t *out_item,
+                                    float *out_score, daisy_stream_t stream);
+
 /* ---- introspection for tests / bench ------------------------------------------------------------- */
 /* Number of kernels launched by this handle since creation (the bench's gpu_launches claim). */
 DAISY_API int daisy_launch_count(daisy_handle_t h, int64_t *n);

@@ -125,6 +125,9 @@ SIGNATURES = {
     "daisy_neumf_scratch_bytes": [ctypes.POINTER(NeuMFParams), c_i64, ctypes.POINTER(c_i64)],
     "daisy_neumf_forward": [c_vp, ctypes.POINTER(NeuMFParams), c_vp, c_i64, c_vp, c_vp],
     "daisy_neumf_step": [c_vp, ctypes.POINTER(NeuMFParams), c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp],
+    "daisy_neumf_topk_candidates": [c_vp, ctypes.POINTER(NeuMFParams), c_vp, c_vp, c_i64, c_i32, c_i32, c_vp, c_vp, c_vp,
+                                    c_vp],
+    "daisy_neumf_topk_full": [c_vp, ctypes.POINTER(NeuMFParams), c_vp, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp],
     "daisy_launch_count": [c_vp, ctypes.POINTER(c_i64)],
     "daisy_set_timing": [c_vp, c_i32],
     "daisy_last_step_timing": [c_vp, ctypes.POINTER(c_f32), ctypes.POINTER(c_f32)],

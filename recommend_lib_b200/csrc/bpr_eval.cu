@@ -7,6 +7,7 @@
 #include <float.h>
 
 #include "ctx.cuh"
+#include "topk_cand.cuh"
 
 namespace {
 
@@ -47,26 +48,6 @@ __global__ void __launch_bounds__(256) k_forward(const float *__restrict__ P, co
 // ------------------------------------------------------------------------------------------------
 // candidate-list top-K: one block per (user, candidate list) group
 // ------------------------------------------------------------------------------------------------
-struct Best {
-    float v;
-    int idx;
-};
-__device__ __forceinline__ bool better(float v, int idx, float bv, int bidx) {
-    return (v > bv) || (v == bv && idx < bidx);  // score desc, position asc
-}
-__device__ __forceinline__ Best warp_best(Best b) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float ov = __shfl_xor_sync(0xffffffffu, b.v, o);
-        const int oi = __shfl_xor_sync(0xffffffffu, b.idx, o);
-        if (better(ov, oi, b.v, b.idx)) {
-            b.v = ov;
-            b.idx = oi;
-        }
-    }
-    return b;
-}
-
 __global__ void __launch_bounds__(256) k_topk_cand(const float *__restrict__ P, const float *__restrict__ Q,
                                                     const int32_t *__restrict__ users,
                                                     const int32_t *__restrict__ cand, int N, int C, int K, uint32_t U,
@@ -74,8 +55,6 @@ __global__ void __launch_bounds__(256) k_topk_cand(const float *__restrict__ P, 
                                                     int32_t *__restrict__ out_item, float *__restrict__ out_score,
                                                     int *err) {
     extern __shared__ float sc[];  // [C] scores of the current group
-    __shared__ Best wbest[8];
-    __shared__ int s_win;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     for (int n = blockIdx.x; n < N; n += gridDim.x) {
         uint32_t u = (uint32_t)users[n];
@@ -118,45 +97,7 @@ __global__ void __launch_bounds__(256) k_topk_cand(const float *__restrict__ P, 
             }
         }
         __syncthreads();
-        // K rounds of block arg-best; a taken entry is marked with -inf and an index flag
-        for (int k = 0; k < K; ++k) {
-            Best b;
-            b.v = -INFINITY;
-            b.idx = 0x7fffffff;
-            for (int c = threadIdx.x; c < C; c += 256) {
-                const float v = sc[c];
-                if (!(v != v) && better(v, c, b.v, b.idx) && v != -INFINITY) {
-                    b.v = v;
-                    b.idx = c;
-                }
-            }
-            b = warp_best(b);
-            if (lane == 0) wbest[wid] = b;
-            __syncthreads();
-            if (wid == 0) {
-                Best t = (lane < 8) ? wbest[lane] : Best{-INFINITY, 0x7fffffff};
-                t = warp_best(t);
-                if (lane == 0) {
-                    int w = t.idx;
-                    if (w == 0x7fffffff) {  // only -inf / NaN scores left: take the lowest untaken position
-                        w = -1;
-                    }
-                    s_win = w;
-                    if (w >= 0) {
-                        out_pos[(size_t)n * K + k] = w;
-                        out_item[(size_t)n * K + k] = cn[w];
-                        out_score[(size_t)n * K + k] = t.v;
-                    } else {
-                        out_pos[(size_t)n * K + k] = -1;
-                        out_item[(size_t)n * K + k] = -1;
-                        out_score[(size_t)n * K + k] = -INFINITY;
-                    }
-                }
-            }
-            __syncthreads();
-            if (threadIdx.x == 0 && s_win >= 0) sc[s_win] = -INFINITY;
-            __syncthreads();
-        }
+        topk_cand_rounds(sc, C, K, cn, out_pos + (size_t)n * K, out_item + (size_t)n * K, out_score + (size_t)n * K);
     }
 }
 

@@ -8,11 +8,14 @@ Ranking order is (score desc, candidate position asc) -- ``torch.topk`` leaves t
 """
 from __future__ import annotations
 
+import ctypes
+
 import numpy as np
 import torch
 
 from . import _lib
 from ._lib import c_vp
+from .ncf_mlp import NeuMF
 
 
 def _i32(x, device):
@@ -20,21 +23,29 @@ def _i32(x, device):
 
 
 def topk_candidates(model, users, cands, top_k):
-    """users [N], cands [N, C] -> (pos [N,K] candidate positions, items [N,K], scores [N,K]) as device tensors."""
-    P, Q = model._tables()
-    users = _i32(users, P.device).reshape(-1)
-    cands = _i32(cands, P.device)
+    """users [N], cands [N, C] -> (pos [N,K] candidate positions, items [N,K], scores [N,K]) as device tensors.
+    ``model``: a dot-product model with ``_tables()`` (BPR, NCF(model='GMF')) or a ``NeuMF`` ('MLP' / 'NeuMF-end'),
+    whose tower scores rank through ``daisy_neumf_topk_candidates``."""
+    neumf = isinstance(model, NeuMF)
+    dev = model._device() if neumf else model._tables()[0].device
+    users = _i32(users, dev).reshape(-1)
+    cands = _i32(cands, dev)
     N, C = cands.shape
     if users.shape[0] != N:
         raise ValueError("users and cands disagree on the number of groups")
     h = model.handle()
-    pos = torch.empty((N, top_k), dtype=torch.int32, device=P.device)
-    items = torch.empty((N, top_k), dtype=torch.int32, device=P.device)
-    scores = torch.empty((N, top_k), dtype=torch.float32, device=P.device)
-    _lib.check(h.L.daisy_topk_candidates(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()),
-                                         c_vp(cands.data_ptr()), N, C, int(top_k), c_vp(pos.data_ptr()),
-                                         c_vp(items.data_ptr()), c_vp(scores.data_ptr()),
-                                         _lib.stream_ptr(torch, P.device)))
+    pos = torch.empty((N, top_k), dtype=torch.int32, device=dev)
+    items = torch.empty((N, top_k), dtype=torch.int32, device=dev)
+    scores = torch.empty((N, top_k), dtype=torch.float32, device=dev)
+    out = (c_vp(pos.data_ptr()), c_vp(items.data_ptr()), c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev))
+    if neumf:
+        prm = model.params()
+        _lib.check(h.L.daisy_neumf_topk_candidates(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()),
+                                                   c_vp(cands.data_ptr()), N, C, int(top_k), *out))
+    else:
+        P, Q = model._tables()
+        _lib.check(h.L.daisy_topk_candidates(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()),
+                                             c_vp(cands.data_ptr()), N, C, int(top_k), *out))
     model.check()
     return pos, items, scores
 
@@ -51,10 +62,12 @@ def hr_ndcg(pos):
 
 def metric_eval(model, test_loader, top_k, algo="bpr"):
     """Drop-in for ``metric_eval`` (util/metrics.py:88-94); returns (HR, NDCG).  ``algo='bpr'`` (``_bpr_topk``) with a
-    ``BPR`` model, ``algo='ncf'`` (``_ncf_topk``, :68-86) with an ``NCF(model='GMF')`` model: both loaders yield
+    ``BPR`` model, ``algo='ncf'`` (``_ncf_topk``, :68-86) with an ``NCF(model='GMF')`` or a ``NeuMF`` model: both loaders yield
     (user, candidates, _) groups whose first candidate is the ground truth."""
     if algo not in ("bpr", "ncf"):
         raise ValueError("algo must be 'bpr' or 'ncf'")
+    if algo == "bpr" and isinstance(model, NeuMF):   # _bpr_topk calls model(user, item_i, item_j), which NCF does not take
+        raise ValueError("algo='bpr' needs a BPR model; rank an NCF model with algo='ncf'")
     groups = {}
     order = []
     for user, item_i, _ in test_loader:
@@ -83,25 +96,31 @@ def metric_eval(model, test_loader, top_k, algo="bpr"):
 def topk_full(model, users, k, exclude=None):
     """Full-catalogue top-k for ``users``: (items [N,k] int32, scores [N,k]) device tensors, order (score desc, item asc).
     ``exclude``: optional per-user lists of item ids to mask (training positives)."""
-    P, Q = model._tables()
-    users = _i32(users, P.device).reshape(-1)
+    neumf = isinstance(model, NeuMF)
+    dev = model._device() if neumf else model._tables()[0].device
+    users = _i32(users, dev).reshape(-1)
     N = users.shape[0]
     h = model.handle()
-    items = torch.empty((N, k), dtype=torch.int32, device=P.device)
-    scores = torch.empty((N, k), dtype=torch.float32, device=P.device)
+    items = torch.empty((N, k), dtype=torch.int32, device=dev)
+    scores = torch.empty((N, k), dtype=torch.float32, device=dev)
     ptr_t = idx_t = None
     if exclude is not None:
         lens = np.fromiter((len(e) for e in exclude), dtype=np.int64, count=N)
         ptr = np.zeros(N + 1, dtype=np.int64)
         np.cumsum(lens, out=ptr[1:])
         idx = np.concatenate([np.asarray(e, dtype=np.int32) for e in exclude]) if ptr[-1] else np.zeros(0, np.int32)
-        ptr_t = torch.from_numpy(ptr).to(P.device)
-        idx_t = torch.from_numpy(idx).to(P.device)
-    _lib.check(h.L.daisy_topk_full(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()), N, int(k),
-                                   c_vp(ptr_t.data_ptr()) if ptr_t is not None else None,
-                                   c_vp(idx_t.data_ptr()) if idx_t is not None and idx_t.numel() else None,
-                                   c_vp(items.data_ptr()), c_vp(scores.data_ptr()),
-                                   _lib.stream_ptr(torch, P.device)))
+        ptr_t = torch.from_numpy(ptr).to(dev)
+        idx_t = torch.from_numpy(idx).to(dev)
+    excl = (c_vp(ptr_t.data_ptr()) if ptr_t is not None else None,
+            c_vp(idx_t.data_ptr()) if idx_t is not None and idx_t.numel() else None)
+    out = (c_vp(items.data_ptr()), c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev))
+    if neumf:
+        prm = model.params()
+        _lib.check(h.L.daisy_neumf_topk_full(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()), N, int(k), *excl, *out))
+    else:
+        P, Q = model._tables()
+        _lib.check(h.L.daisy_topk_full(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()), N, int(k),
+                                       *excl, *out))
     model.check()
     return items, scores
 
