@@ -386,6 +386,14 @@ DAISY_API int daisy_fmbn_step(daisy_handle_t h, const daisy_fmbn_params *p, cons
  * the user bias and bias_ (equal for every item of a user). */
 DAISY_API int daisy_fmbn_forward(daisy_handle_t h, const daisy_fmbn_params *p, const int32_t *triples, int64_t B,
                        float *pred_i, float *pred_j, daisy_stream_t stream);
+/* Ranking tables of the evaluation-mode model (BPRFMRecommender.py:57-80 after model.eval()): with
+ * a_f = gamma_f / sqrt(running_var_f + bn_eps), P_out [user_num, W] = [a (.) e_u, 1, 0...], Q_out [item_num, W] =
+ * [e_i, b_i, 0...] and *c0_out = sum_f (beta_f - a_f running_mean_f), so that the forward score is
+ * <P[u], Q[i]> + b_u + bias_ + c0.  W % 4 == 0, W >= F + 1 (the 16-byte rows of the ranking kernels); rank with
+ * daisy_topk_candidates / daisy_topk_full on a handle of dim W, then add b_u + bias_ + c0 per user.  Only the forward
+ * fields of p are read.  Deterministic: the same bits on every call. */
+DAISY_API int daisy_fmbn_rank_tables(daisy_handle_t h, const daisy_fmbn_params *p, int W, float *P_out, float *Q_out,
+                                     float *c0_out, daisy_stream_t stream);
 
 /* ---- Item2Vec / skip-gram with negative sampling (SURVEY section 8f, row N4) ---------------------------------------
  * GPU-verified in round 2 (tests/test_sgns_gpu.py).

@@ -119,6 +119,7 @@ SIGNATURES = {
     "daisy_fmbn_scratch_bytes": [c_i64, c_i32, ctypes.POINTER(c_i64)],
     "daisy_fmbn_step": [c_vp, ctypes.POINTER(FMBNParams), c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp],
     "daisy_fmbn_forward": [c_vp, ctypes.POINTER(FMBNParams), c_vp, c_i64, c_vp, c_vp, c_vp],
+    "daisy_fmbn_rank_tables": [c_vp, ctypes.POINTER(FMBNParams), c_i32, c_vp, c_vp, c_vp, c_vp],
     "daisy_sgns_scratch_bytes": [c_i64, c_i32, c_i32, c_i64, c_i32, ctypes.POINTER(c_i64)],
     "daisy_sgns_step": [c_vp, ctypes.POINTER(SGNSParams), c_vp, c_vp, c_vp, c_i64, c_i32, c_i32, c_i64, c_vp, c_i64, c_vp,
                         c_vp],

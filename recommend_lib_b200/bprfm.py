@@ -138,6 +138,13 @@ class BPRFM(nn.Module):
         extra = self.biases.weight[tri[:, 0].long(), 0] + self.bias_          # user bias + global bias: the same in both
         return (pi + extra).view(-1), (pj + extra).view(-1)
 
+    def rank_tables(self):
+        """(P, Q, None): the augmented rows the library trains on, so that ``forward()``'s score is
+        <P[u], Q[i]> + b_u + bias_.  Views of the training buffer: no copy, and unsynced training is included."""
+        if self._aug is None:
+            self.pack()
+        return self._aug, self._aug[self.user_num:], None
+
     def state_dict(self, *args, **kwargs):
         self.sync()
         return super().state_dict(*args, **kwargs)

@@ -1,5 +1,6 @@
 """BPR-FM at the reference script's DEFAULTS -- batch norm + dropout on the FM vector (BPRFMRecommender.py:45-80, 116-125)
--- on the C-ABI library (``daisy_fmbn_step`` / ``daisy_fmbn_forward``, csrc/fmbn.cu).  SURVEY.md section 8f, row N3.
+-- on the C-ABI library (``daisy_fmbn_step`` / ``daisy_fmbn_forward``, and ``daisy_fmbn_rank_tables`` for ranking;
+csrc/fmbn.cu).  SURVEY.md section 8f, row N3.
 
 ``bprfm.BPRFM(batch_norm=True, ...)`` builds this class (and ``FMAdagrad`` on it the optimiser below), so the reference's
 one constructor covers both configurations.  Parity: tests/test_bprfm_bn_gpu.py against the golden run of the unmodified
@@ -64,8 +65,9 @@ class BPRFMBN(nn.Module):
         if h is None or h.device_index != idx:
             if h is not None:
                 h.close()
-            # the handle only carries the device, the error flag and the launch counter for this path
-            h = _lib.Handle(idx, self.user_num, self.item_num, 4, 0)
+            # the step and the forward read the device, the error flag and the launch counter; the ranking entry points
+            # also read the row width of the folded tables (rank_tables)
+            h = _lib.Handle(idx, self.user_num, self.item_num, self.rank_width, 0)
             self._handle = h
         return h
 
@@ -117,6 +119,28 @@ class BPRFMBN(nn.Module):
                                           c_vp(pj.data_ptr()), _lib.stream_ptr(torch, dev)))
         extra = self.biases.weight[tri[:, 0].long(), 0] + self.bias_          # user bias + global bias: the same in both
         return (pi + extra).view(-1), (pj + extra).view(-1)
+
+    @property
+    def rank_width(self):
+        """Row width W of the ranking tables: F + 1 rounded up to a multiple of 4 (the ranking kernels read 16-byte rows)."""
+        return (self.num_factors + 4) // 4 * 4
+
+    def rank_tables(self):
+        """(P [user_num, W], Q [item_num, W], c0 [1]): the evaluation-mode score folded into a dot product,
+        ``forward()``'s score = <P[u], Q[i]> + b_u + bias_ + c0 (``daisy_fmbn_rank_tables``).  Folded anew on every call,
+        since training moves the weights and the running statistics."""
+        if self.training:
+            raise RuntimeError("training-mode forward is fused into FMBNAdagrad.step; call model.eval() to predict")
+        dev = self._device()
+        h = self.handle()
+        W = self.rank_width
+        P = torch.empty((self.user_num, W), dtype=torch.float32, device=dev)
+        Q = torch.empty((self.item_num, W), dtype=torch.float32, device=dev)
+        c0 = torch.empty(1, dtype=torch.float32, device=dev)
+        prm = self.params()
+        _lib.check(h.L.daisy_fmbn_rank_tables(h.ptr, ctypes.byref(prm), W, c_vp(P.data_ptr()), c_vp(Q.data_ptr()),
+                                              c_vp(c0.data_ptr()), _lib.stream_ptr(torch, dev)))
+        return P, Q, c0
 
     def __getstate__(self):
         d = self.__dict__.copy()

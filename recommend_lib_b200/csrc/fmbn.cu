@@ -451,6 +451,39 @@ __global__ void __launch_bounds__(256) k_fm_forward(const float *__restrict__ E,
     }
 }
 
+// Ranking tables of the evaluation-mode model, one warp per row.  With a_f = gamma_f / sqrt(rvar_f + bn_eps) the score
+// of k_fm_forward is sum_f a_f e_u,f e_i,f + b_i + (b_u + bias_ + C0), C0 = sum_f (beta_f - a_f mu_f); the rows
+// P[u] = [a (.) e_u, 1, 0...] and Q[i] = [e_i, b_i, 0...] make the first two terms a dot product, so the ranking kernels
+// of bpr_eval.cu / topk_full.cu rank them unchanged.  a_f is formed as k_fm_forward forms its factors.  C0 is summed by
+// one thread in ascending f: the same bits on every call.
+__global__ void __launch_bounds__(256) k_fm_rank_rows(const float *__restrict__ E, const float *__restrict__ bias,
+                                                       int64_t rows, int64_t U, int F, int W,
+                                                       const float *__restrict__ gamma, const float *__restrict__ beta,
+                                                       const float *__restrict__ rmean, const float *__restrict__ rvar,
+                                                       float bn_eps, float *__restrict__ P, float *__restrict__ Q,
+                                                       float *__restrict__ c0) {
+    const int lane = threadIdx.x & 31;
+    const int64_t r = (int64_t)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
+    if (r == 0 && lane == 0) {
+        double c = 0.0;
+        for (int f = 0; f < F; ++f) {
+            const float a = gamma[f] * (1.f / sqrtf(rvar[f] + bn_eps));
+            c += (double)beta[f] - (double)a * (double)rmean[f];
+        }
+        *c0 = (float)c;
+    }
+    if (r >= rows) return;
+    const float *e = E + (size_t)r * F;
+    if (r < U) {
+        float *p = P + (size_t)r * W;
+        for (int f = lane; f < W; f += 32)
+            p[f] = f < F ? gamma[f] * (1.f / sqrtf(rvar[f] + bn_eps)) * e[f] : (f == F ? 1.f : 0.f);
+    } else {
+        float *q = Q + (size_t)(r - U) * W;
+        for (int f = lane; f < W; f += 32) q[f] = f < F ? e[f] : (f == F ? bias[r] : 0.f);
+    }
+}
+
 static int fm_check(daisy_ctx *h, const daisy_fmbn_params *p, const void *triples, int64_t B) {
     DAISY_REQUIRE(h != nullptr && p != nullptr, DAISY_EINVAL, "null handle or parameter block");
     DAISY_REQUIRE(p->E && p->bias && p->gamma && p->beta && p->running_mean && p->running_var, DAISY_EINVAL,
@@ -542,6 +575,22 @@ extern "C" int daisy_fmbn_forward(daisy_handle_t h, const daisy_fmbn_params *p, 
     k_fm_forward<<<daisy_ceil_div(B, 8), 256, 0, s>>>(p->E, p->bias, triples, (int)B, p->F, (uint32_t)p->user_num,
                                                       (uint32_t)(p->num_features - p->user_num), p->gamma, p->beta,
                                                       p->running_mean, p->running_var, p->bn_eps, pred_i, pred_j, h->err);
+    DAISY_LAUNCH_CHECK(h);
+    return DAISY_OK;
+}
+
+extern "C" int daisy_fmbn_rank_tables(daisy_handle_t h, const daisy_fmbn_params *p, int W, float *P_out, float *Q_out,
+                                      float *c0_out, daisy_stream_t stream) {
+    int rc = fm_check(h, p, nullptr, 0);
+    if (rc) return rc;
+    DAISY_REQUIRE(W >= p->F + 1 && W % 4 == 0, DAISY_EINVAL, "row width %d: need W >= F + 1 = %d and W %% 4 == 0", W, p->F + 1);
+    DAISY_REQUIRE(P_out && Q_out && c0_out, DAISY_EINVAL, "null output");
+    DeviceGuard g(h->device);
+    DAISY_REQUIRE(g.ok, DAISY_ECUDA, "cannot select device %d", h->device);
+    const int64_t rows = p->num_features;
+    k_fm_rank_rows<<<daisy_ceil_div(rows, 8), 256, 0, (cudaStream_t)stream>>>(
+        p->E, p->bias, rows, p->user_num, p->F, W, p->gamma, p->beta, p->running_mean, p->running_var, p->bn_eps, P_out,
+        Q_out, c0_out);
     DAISY_LAUNCH_CHECK(h);
     return DAISY_OK;
 }

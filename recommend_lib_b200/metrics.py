@@ -15,6 +15,8 @@ import torch
 
 from . import _lib
 from ._lib import c_vp
+from .bprfm import BPRFM
+from .bprfm_bn import BPRFMBN
 from .ncf_mlp import NeuMF
 
 
@@ -22,12 +24,30 @@ def _i32(x, device):
     return torch.as_tensor(np.asarray(x) if not torch.is_tensor(x) else x).to(device=device, dtype=torch.int32).contiguous()
 
 
+def _tables(model):
+    """(P, Q, c0) that ``daisy_topk_candidates`` / ``daisy_topk_full`` rank ``model`` with.  A BPR-FM model's score is
+    <P[u], Q[i]> plus a term that is the same for every item of a user (``_user_offsets``); c0 is the batch-norm
+    model's share of that term, None for the other models."""
+    if isinstance(model, (BPRFM, BPRFMBN)):
+        return model.rank_tables()
+    return (*model._tables(), None)
+
+
+def _user_offsets(model, users, c0):
+    """b_u + bias_ (+ c0) per ranked user of a BPR-FM model: what ``forward()`` adds to every item of a user.  Call
+    only after ``model.check()``, so that an out-of-range user id raises there and never reaches this gather."""
+    off = model.biases.weight[users.long(), 0] + model.bias_
+    return off if c0 is None else off + c0
+
+
 def topk_candidates(model, users, cands, top_k):
     """users [N], cands [N, C] -> (pos [N,K] candidate positions, items [N,K], scores [N,K]) as device tensors.
-    ``model``: a dot-product model with ``_tables()`` (BPR, NCF(model='GMF')) or a ``NeuMF`` ('MLP' / 'NeuMF-end'),
-    whose tower scores rank through ``daisy_neumf_topk_candidates``."""
+    ``model``: a dot-product model with ``_tables()`` (BPR, NCF(model='GMF')), a BPR-FM model (``BPRFM``, and
+    ``BPRFM(batch_norm=True)`` in evaluation mode), whose score is folded into one, or a ``NeuMF`` ('MLP' /
+    'NeuMF-end'), whose tower scores rank through ``daisy_neumf_topk_candidates``."""
     neumf = isinstance(model, NeuMF)
-    dev = model._device() if neumf else model._tables()[0].device
+    bprfm = isinstance(model, (BPRFM, BPRFMBN))
+    dev = model._device() if neumf or bprfm else model._tables()[0].device
     users = _i32(users, dev).reshape(-1)
     cands = _i32(cands, dev)
     N, C = cands.shape
@@ -43,10 +63,12 @@ def topk_candidates(model, users, cands, top_k):
         _lib.check(h.L.daisy_neumf_topk_candidates(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()),
                                                    c_vp(cands.data_ptr()), N, C, int(top_k), *out))
     else:
-        P, Q = model._tables()
+        P, Q, c0 = _tables(model)
         _lib.check(h.L.daisy_topk_candidates(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()),
                                              c_vp(cands.data_ptr()), N, C, int(top_k), *out))
     model.check()
+    if bprfm:
+        scores += _user_offsets(model, users, c0)[:, None]
     return pos, items, scores
 
 
@@ -62,8 +84,9 @@ def hr_ndcg(pos):
 
 def metric_eval(model, test_loader, top_k, algo="bpr"):
     """Drop-in for ``metric_eval`` (util/metrics.py:88-94); returns (HR, NDCG).  ``algo='bpr'`` (``_bpr_topk``) with a
-    ``BPR`` model, ``algo='ncf'`` (``_ncf_topk``, :68-86) with an ``NCF(model='GMF')`` or a ``NeuMF`` model: both loaders yield
-    (user, candidates, _) groups whose first candidate is the ground truth."""
+    ``BPR`` model, ``algo='ncf'`` (``_ncf_topk``, :68-86) with an ``NCF(model='GMF')`` or a ``NeuMF`` model; a BPR-FM model
+    (``BPRFM``, or ``BPRFM(batch_norm=True)`` after ``model.eval()``) with either: both loaders yield (user, candidates, _)
+    groups whose first candidate is the ground truth."""
     if algo not in ("bpr", "ncf"):
         raise ValueError("algo must be 'bpr' or 'ncf'")
     if algo == "bpr" and isinstance(model, NeuMF):   # _bpr_topk calls model(user, item_i, item_j), which NCF does not take
@@ -95,9 +118,11 @@ def metric_eval(model, test_loader, top_k, algo="bpr"):
 
 def topk_full(model, users, k, exclude=None):
     """Full-catalogue top-k for ``users``: (items [N,k] int32, scores [N,k]) device tensors, order (score desc, item asc).
+    ``model``: BPR, NCF(model='GMF'), a BPR-FM model or a ``NeuMF``, as for ``topk_candidates``.
     ``exclude``: optional per-user lists of item ids to mask (training positives)."""
     neumf = isinstance(model, NeuMF)
-    dev = model._device() if neumf else model._tables()[0].device
+    bprfm = isinstance(model, (BPRFM, BPRFMBN))
+    dev = model._device() if neumf or bprfm else model._tables()[0].device
     users = _i32(users, dev).reshape(-1)
     N = users.shape[0]
     h = model.handle()
@@ -118,10 +143,12 @@ def topk_full(model, users, k, exclude=None):
         prm = model.params()
         _lib.check(h.L.daisy_neumf_topk_full(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()), N, int(k), *excl, *out))
     else:
-        P, Q = model._tables()
+        P, Q, c0 = _tables(model)
         _lib.check(h.L.daisy_topk_full(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()), N, int(k),
                                        *excl, *out))
     model.check()
+    if bprfm:
+        scores += _user_offsets(model, users, c0)[:, None]
     return items, scores
 
 
