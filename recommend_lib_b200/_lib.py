@@ -4,6 +4,9 @@ from __future__ import annotations
 import ctypes
 import os
 
+import numpy as np
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # DAISY_LIB_VARIANT=<name> loads libdaisy_b200_<name>.so, an experimental build made by build.py with DAISY_NVCC_EXTRA
 _VARIANT = os.environ.get("DAISY_LIB_VARIANT", "")
@@ -300,3 +303,132 @@ class Handle:
         steps = c_i64()
         check(self.L.daisy_phase_ms(self.ptr, arr, NUM_PHASES, ctypes.byref(steps)))
         return dict(zip(PHASES, list(arr))), steps.value
+
+
+class HandleOwner:
+    """A model (or optimiser) that owns one ``Handle``: the device check, the handle's lifecycle and, for the models that
+    rank, the ranking calls of ``metrics.topk_candidates`` / ``topk_full``.
+
+    A subclass names the weight it runs on (``_weight``, and ``_cpu_error`` for that weight on the CPU) and the handle's
+    dims (``_handle_dims``).  With ``_batch_grows`` the handle holds a step workspace of ``_max_batch`` rows and is
+    re-created for a larger batch; otherwise it is light (max_batch 0: device, error flag and launch counter).  Adds no
+    parameter, buffer or submodule to an ``nn.Module``."""
+
+    _handle = None
+    _max_batch = 0
+    _batch_grows = False
+    _handle_flags = 0
+    # metric_eval(algo='bpr') ranks as the reference's _bpr_topk, which scores with model(user, item_i, item_j)
+    bpr_topk = True
+
+    def _device(self):
+        W = self._weight()
+        if not W.is_cuda:
+            require_cuda()
+            raise DaisyError(self._cpu_error)
+        return W.device
+
+    def handle(self, batch=None):
+        """The library handle for the weights' current device; re-created when the device changes or, for a handle with a
+        step workspace, when a larger batch arrives."""
+        dev = self._device()
+        idx = dev.index if dev.index is not None else torch.cuda.current_device()
+        need = max(self._max_batch, int(batch or 0)) if self._batch_grows else 0
+        h = self._handle
+        if h is None or h.device_index != idx or (need and h.max_batch < need):   # a light handle never grows
+            self._close_handle()
+            self._max_batch = need
+            self._handle = h = Handle(idx, *self._handle_dims(), need, self._handle_flags)
+        return h
+
+    def _close_handle(self):
+        if self._handle is not None:
+            self._handle.close()
+            self._handle = None
+
+    def check(self):
+        """Synchronise and raise IndexError if any id seen since the last check was out of range."""
+        h = self._handle
+        if h is not None:
+            check(h.L.daisy_check(h.ptr, stream_ptr(torch, self._device())))
+
+    def __getstate__(self):             # a handle does not pickle: the copy makes its own on first use
+        d = self.__dict__.copy()
+        d["_handle"] = None
+        return d
+
+    def _apply(self, fn, *a, **k):      # .cuda() / .cpu() / .to(): the weights move, the handle is rebuilt lazily
+        self._close_handle()
+        return super()._apply(fn, *a, **k)
+
+    # -- ranking: a dot-product model's score is <P[u], Q[i]> (+ a term that is the same for every item of a user) ------
+    def user_term(self, users, c0):
+        """[N] the score's term that is the same for every item of a user, or None when the score is the dot product."""
+        return None
+
+    def rank_candidates(self, users, cands, top_k):
+        """users [N], cands [N, C] int32 device tensors -> (pos, items, scores) [N, top_k]."""
+        h = self.handle()
+        P, Q, c0 = self.rank_tables()
+        pos, items, scores = call_topk_candidates(h, P.data_ptr(), Q.data_ptr(), users, cands, top_k,
+                                                  stream_ptr(torch, users.device))
+        self.check()                    # before the term's gather: an out-of-range user id raises here
+        off = self.user_term(users, c0)
+        if off is not None:
+            scores += off[:, None]
+        return pos, items, scores
+
+    def rank_full(self, users, k, excl):
+        """users [N] int32 device tensor, excl the ``exclusion_csr`` pair -> (items, scores) [N, k]."""
+        h = self.handle()
+        P, Q, c0 = self.rank_tables()
+        items, scores = call_topk_full(h, P.data_ptr(), Q.data_ptr(), users, k, excl, stream_ptr(torch, users.device))
+        self.check()
+        off = self.user_term(users, c0)
+        if off is not None:
+            scores += off[:, None]
+        return items, scores
+
+
+def call_topk_candidates(h, P, Q, users, cands, top_k, stream):
+    """``daisy_topk_candidates`` over the tables at device addresses P, Q: users [N], cands [N, C] int32 device tensors
+    -> (pos, items, scores) [N, top_k] on the users' device."""
+    N, C = cands.shape
+    pos = torch.empty((N, top_k), dtype=torch.int32, device=users.device)
+    items = torch.empty((N, top_k), dtype=torch.int32, device=users.device)
+    scores = torch.empty((N, top_k), dtype=torch.float32, device=users.device)
+    check(h.L.daisy_topk_candidates(h.ptr, c_vp(P), c_vp(Q), c_vp(users.data_ptr()), c_vp(cands.data_ptr()), N, C,
+                                    int(top_k), c_vp(pos.data_ptr()), c_vp(items.data_ptr()), c_vp(scores.data_ptr()),
+                                    stream))
+    return pos, items, scores
+
+
+def call_topk_full(h, P, Q, users, k, excl, stream):
+    """``daisy_topk_full`` over the tables at device addresses P, Q: users [N] int32 device tensor, excl the
+    ``exclusion_csr`` pair -> (items, scores) [N, k] on the users' device."""
+    N = users.shape[0]
+    ptr, idx = excl
+    items = torch.empty((N, k), dtype=torch.int32, device=users.device)
+    scores = torch.empty((N, k), dtype=torch.float32, device=users.device)
+    check(h.L.daisy_topk_full(h.ptr, c_vp(P), c_vp(Q), c_vp(users.data_ptr()), N, int(k),
+                              c_vp(ptr.data_ptr()) if ptr is not None else None,
+                              c_vp(idx.data_ptr()) if idx is not None and idx.numel() else None,
+                              c_vp(items.data_ptr()), c_vp(scores.data_ptr()), stream))
+    return items, scores
+
+
+def exclusion_csr(exclude, n, device, window=None):
+    """(ptr [n + 1] int64, idx int32) on ``device``: the n per-user lists of item ids ``exclude`` as CSR, or (None, None)
+    without lists.  ``window=(i0, i1)`` keeps the ids in [i0, i1), made relative to i0 (one shard of the item table)."""
+    if exclude is None:
+        return None, None
+    if window is None:
+        ex = [np.asarray(e, dtype=np.int32) for e in exclude]
+    else:
+        i0, i1 = window
+        ex = [np.asarray(e, dtype=np.int64) for e in exclude]
+        ex = [(e[(e >= i0) & (e < i1)] - i0).astype(np.int32) for e in ex]
+    ptr = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(np.fromiter((len(e) for e in ex), dtype=np.int64, count=n), out=ptr[1:])
+    idx = np.concatenate(ex) if ptr[-1] else np.zeros(0, np.int32)
+    return torch.from_numpy(ptr).to(device), torch.from_numpy(idx).to(device)

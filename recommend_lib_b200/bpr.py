@@ -35,8 +35,11 @@ def _as_triples(user, item_i, item_j, device):
     return t.to(device=device, dtype=torch.int32, non_blocking=True).contiguous()
 
 
-class BPR(nn.Module):
+class BPR(_lib.HandleOwner, nn.Module):
     """Drop-in for ``class BPR`` (BPRMFRecommender.py:28-50)."""
+
+    _batch_grows = True
+    _cpu_error = "BPR tables are on the CPU: call model.cuda() first (no CPU fallback)"
 
     def __init__(self, user_num, item_num, factor_num, max_batch=4096, eager_decay=False):
         super().__init__()
@@ -47,34 +50,40 @@ class BPR(nn.Module):
         self.user_num, self.item_num, self.factor_num = int(user_num), int(item_num), int(factor_num)
         self._max_batch = int(max_batch)
         self._eager = bool(eager_decay)
-        self._handle = None
         self._pending_scale = 1.0
 
     # -- library plumbing ---------------------------------------------------------------------
-    def _tables(self):
+    def _weight(self):
         # straight from _modules: the attribute route (__getattr__ below) would fold the lazy decay in on every step
-        P, Q = self._modules["embed_user"].weight, self._modules["embed_item"].weight
-        if not P.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("BPR tables are on the CPU: call model.cuda() first (no CPU fallback)")
-        return P, Q
+        return self._modules["embed_user"].weight
+
+    def _handle_dims(self):
+        return self.user_num, self.item_num, self.factor_num
+
+    @property
+    def _handle_flags(self):
+        return _lib.FLAG_EAGER_DECAY if self._eager else 0
+
+    def _tables(self):
+        self._device()
+        return self._modules["embed_user"].weight, self._modules["embed_item"].weight
+
+    def rank_tables(self):
+        return (*self._tables(), None)
 
     def handle(self, batch=None):
-        """The library handle for the tables' current device; re-created when a larger batch arrives."""
-        P, _ = self._tables()
-        dev = P.device.index if P.device.index is not None else torch.cuda.current_device()
-        need = max(self._max_batch, int(batch or 0))
+        """The library handle for the tables' current device; re-created when a larger batch arrives, with the lazy
+        decay scale of the handle it replaces."""
         h = self._handle
-        if h is None or h.device_index != dev or h.max_batch < need:
-            scale = h.scale if h is not None else self._pending_scale
-            if h is not None:
-                h.close()
-            self._max_batch = need
-            h = _lib.Handle(dev, self.user_num, self.item_num, self.factor_num, need,
-                            _lib.FLAG_EAGER_DECAY if self._eager else 0)
-            h.scale = scale
-            self._handle = h
-        return h
+        new = super().handle(batch)
+        if new is not h:
+            new.scale = self._pending_scale
+        return new
+
+    def _close_handle(self):
+        if self._handle is not None:
+            self._pending_scale = self._handle.scale
+        super()._close_handle()
 
     @property
     def decay_scale(self):
@@ -102,12 +111,6 @@ class BPR(nn.Module):
         _lib.check(h.L.daisy_set_l2_window(h.ptr, c_vp(Q.data_ptr()), n, float(hit_ratio),
                                            _lib.stream_ptr(torch, P.device)))
         return self
-
-    def check(self):
-        """Synchronise and raise IndexError if any id seen since the last check was out of range."""
-        if self._handle is not None:
-            P, _ = self._tables()
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, P.device)))
 
     # -- reference surface --------------------------------------------------------------------
     def forward(self, user, item_i, item_j):
@@ -156,16 +159,12 @@ class BPR(nn.Module):
 
     def __getstate__(self):
         self.materialize()
-        d = self.__dict__.copy()
-        d["_handle"] = None
+        d = super().__getstate__()
         d["_pending_scale"] = 1.0
         return d
 
-    def _apply(self, fn, *a, **k):          # .cuda() / .cpu() / .to(): weights move, the handle is rebuilt lazily
-        if self._handle is not None:
-            self.materialize()
-            self._handle.close()
-            self._handle = None
+    def _apply(self, fn, *a, **k):
+        self.materialize()
         return super()._apply(fn, *a, **k)
 
 

@@ -20,7 +20,7 @@ from . import _lib
 c_vp = ctypes.c_void_p
 
 
-class BPRFM(nn.Module):
+class BPRFM(_lib.HandleOwner, nn.Module):
     """``BPRFM(num_features, num_factors, batch_norm, drop_prob, user_num=...)``: attributes ``embeddings``, ``biases``,
     ``bias_`` as in the reference (:45-55).  ``user_num`` (features ``[0, user_num)`` are users, the rest items) is the
     one extra argument the accelerated path needs.
@@ -29,6 +29,9 @@ class BPRFM(nn.Module):
     that the bias term and its gradient ride through the BPR kernels; ``embeddings.weight`` / ``biases.weight`` are
     refreshed from that buffer whenever they are read through ``forward``, ``state_dict`` or ``sync()``.
     """
+
+    _batch_grows = True
+    _cpu_error = "BPRFM tables are on the CPU: call model.cuda() first (no CPU fallback)"
 
     def __new__(cls, num_features=None, num_factors=None, batch_norm=False, drop_prob=(0.0, 0.0), *args, **kwargs):
         # the reference has ONE class (BPRFMRecommender.py:29-55) and the script's defaults are batch_norm=True,
@@ -58,18 +61,16 @@ class BPRFM(nn.Module):
         for p in self.parameters():
             p.requires_grad_(False)
         self._max_batch = int(max_batch)
-        self._handle = None
         self._aug = None        # [num_features, F + 4] device buffer the library trains on
         self._dirty = False     # _aug is newer than embeddings / biases
 
-    # -- augmented layout ---------------------------------------------------------------------------------------------
-    def _device(self):
-        E = self.embeddings.weight
-        if not E.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("BPRFM tables are on the CPU: call model.cuda() first (no CPU fallback)")
-        return E.device
+    def _weight(self):
+        return self.embeddings.weight
 
+    def _handle_dims(self):
+        return self.user_num, self.item_num, self.num_factors + 4
+
+    # -- augmented layout ---------------------------------------------------------------------------------------------
     def pack(self):
         """Build the augmented buffer from embeddings / biases (after the weights were set from outside)."""
         dev = self._device()
@@ -90,23 +91,6 @@ class BPRFM(nn.Module):
                 self.biases.weight[U:, 0] = self._aug[U:, F]
             self._dirty = False
         return self
-
-    def handle(self, batch=None):
-        dev = self._device()
-        idx = dev.index if dev.index is not None else torch.cuda.current_device()
-        need = max(self._max_batch, int(batch or 0))
-        h = self._handle
-        if h is None or h.device_index != idx or h.max_batch < need:
-            if h is not None:
-                h.close()
-            self._max_batch = need
-            h = _lib.Handle(idx, self.user_num, self.item_num, self.num_factors + 4, need, 0)
-            self._handle = h
-        return h
-
-    def check(self):
-        if self._handle is not None:
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, self._device())))
 
     def triples(self, features_i, feature_values_i, features_j, feature_values_j):
         """(user, item_i, item_j) int32 [B,3] on the device from the loader's tensors; validates the feature layout."""
@@ -145,21 +129,24 @@ class BPRFM(nn.Module):
             self.pack()
         return self._aug, self._aug[self.user_num:], None
 
+    def user_term(self, users, c0):
+        """b_u + bias_ (+ c0) per ranked user: what ``forward()`` adds to every item of a user (c0: the batch-norm model's
+        share, ``BPRFMBN.rank_tables``).  Gathers by user id, so call it only after ``check()``."""
+        off = self.biases.weight[users.long(), 0] + self.bias_
+        return off if c0 is None else off + c0
+
     def state_dict(self, *args, **kwargs):
         self.sync()
         return super().state_dict(*args, **kwargs)
 
     def __getstate__(self):
         self.sync()
-        d = self.__dict__.copy()
-        d["_handle"], d["_aug"], d["_dirty"] = None, None, False
+        d = super().__getstate__()
+        d["_aug"], d["_dirty"] = None, False
         return d
 
     def _apply(self, fn, *a, **k):
         self.sync()
-        if self._handle is not None:
-            self._handle.close()
-            self._handle = None
         self._aug = None
         return super()._apply(fn, *a, **k)
 

@@ -19,12 +19,16 @@ import torch
 import torch.nn as nn
 
 from . import _lib
+from .bprfm import BPRFM
 
 c_vp = ctypes.c_void_p
 
 
-class BPRFMBN(nn.Module):
+class BPRFMBN(_lib.HandleOwner, nn.Module):
     """``BPRFM(num_features, num_factors, batch_norm=True, drop_prob, user_num=...)`` (BPRFMRecommender.py:29-55)."""
+
+    _cpu_error = "BPRFMBN tables are on the CPU: call model.cuda() first (no CPU fallback)"
+    user_term = BPRFM.user_term
 
     def __init__(self, num_features, num_factors, batch_norm=True, drop_prob=(0.5, 0.2), user_num=None, max_batch=4096):
         super().__init__()
@@ -47,33 +51,15 @@ class BPRFMBN(nn.Module):
         nn.init.constant_(self.biases.weight, 0.0)
         for p in self.parameters():
             p.requires_grad_(False)
-        self._max_batch = int(max_batch)
-        self._handle = None
 
     # -- plumbing -----------------------------------------------------------------------------------------------------
-    def _device(self):
-        E = self.embeddings.weight
-        if not E.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("BPRFMBN tables are on the CPU: call model.cuda() first (no CPU fallback)")
-        return E.device
+    def _weight(self):
+        return self.embeddings.weight
 
-    def handle(self):
-        dev = self._device()
-        idx = dev.index if dev.index is not None else torch.cuda.current_device()
-        h = self._handle
-        if h is None or h.device_index != idx:
-            if h is not None:
-                h.close()
-            # the step and the forward read the device, the error flag and the launch counter; the ranking entry points
-            # also read the row width of the folded tables (rank_tables)
-            h = _lib.Handle(idx, self.user_num, self.item_num, self.rank_width, 0)
-            self._handle = h
-        return h
-
-    def check(self):
-        if self._handle is not None:
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, self._device())))
+    def _handle_dims(self):
+        # the step and the forward read the device, the error flag and the launch counter; the ranking entry points
+        # also read the row width of the folded tables (rank_tables)
+        return self.user_num, self.item_num, self.rank_width
 
     def params(self, lr=0.0, eps=1e-10, state=None):
         """The ``daisy_fmbn_params`` block over this module's tensors (+ an optimizer's state_sum tensors)."""
@@ -141,17 +127,6 @@ class BPRFMBN(nn.Module):
         _lib.check(h.L.daisy_fmbn_rank_tables(h.ptr, ctypes.byref(prm), W, c_vp(P.data_ptr()), c_vp(Q.data_ptr()),
                                               c_vp(c0.data_ptr()), _lib.stream_ptr(torch, dev)))
         return P, Q, c0
-
-    def __getstate__(self):
-        d = self.__dict__.copy()
-        d["_handle"] = None
-        return d
-
-    def _apply(self, fn, *a, **k):
-        if self._handle is not None:
-            self._handle.close()
-            self._handle = None
-        return super()._apply(fn, *a, **k)
 
 
 class FMBNAdagrad:

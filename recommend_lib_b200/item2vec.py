@@ -70,10 +70,12 @@ class SGNS(nn.Module):
         raise RuntimeError("the SGNS loss, its backward and the Adam step are fused: use SGNSAdam(sgns).step(iword, owords)")
 
 
-class SGNSAdam:
+class SGNSAdam(_lib.HandleOwner):
     """``optim.Adam(sgns.parameters())`` (:266) + the step of :274-277, fused: ``step(iword, owords, nwords=None)``.
     ``nwords`` ([B, C * n_negs]) replaces the draw inside the reference's forward -- that is how the parity tests feed the
     negatives the reference drew; without it they are drawn on the device (``SGNS.draw_negatives``)."""
+
+    _cpu_error = "Item2Vec tables are on the CPU: call sgns.cuda() first (no CPU fallback)"
 
     def __init__(self, sgns: SGNS, lr=1e-3, betas=(0.9, 0.999), eps=1e-8):
         self.sgns, self.lr, self.betas, self.eps = sgns, float(lr), (float(betas[0]), float(betas[1])), float(eps)
@@ -81,28 +83,13 @@ class SGNSAdam:
         self.state = None
         self._scratch = None
         self._loss = None
-        self._handle = None
 
-    def _device(self):
-        W = self.sgns.embedding.ivectors.weight
-        if not W.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("Item2Vec tables are on the CPU: call sgns.cuda() first (no CPU fallback)")
-        return W.device
+    def _weight(self):
+        return self.sgns.embedding.ivectors.weight
 
-    def handle(self):
-        dev = self._device()
-        idx = dev.index if dev.index is not None else torch.cuda.current_device()
-        if self._handle is None or self._handle.device_index != idx:
-            if self._handle is not None:
-                self._handle.close()
-            V = self.sgns.embedding.vocab_size
-            self._handle = _lib.Handle(idx, V, V, 4, 0)     # carries the device, the error flag and the launch counter
-        return self._handle
-
-    def check(self):
-        if self._handle is not None:
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, self._device())))
+    def _handle_dims(self):
+        V = self.sgns.embedding.vocab_size
+        return V, V, 4                                  # carries the device, the error flag and the launch counter
 
     def step(self, iword, owords, nwords=None):
         emb = self.sgns.embedding

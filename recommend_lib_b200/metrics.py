@@ -8,68 +8,28 @@ Ranking order is (score desc, candidate position asc) -- ``torch.topk`` leaves t
 """
 from __future__ import annotations
 
-import ctypes
-
 import numpy as np
 import torch
 
 from . import _lib
-from ._lib import c_vp
-from .bprfm import BPRFM
-from .bprfm_bn import BPRFMBN
-from .ncf_mlp import NeuMF
 
 
 def _i32(x, device):
     return torch.as_tensor(np.asarray(x) if not torch.is_tensor(x) else x).to(device=device, dtype=torch.int32).contiguous()
 
 
-def _tables(model):
-    """(P, Q, c0) that ``daisy_topk_candidates`` / ``daisy_topk_full`` rank ``model`` with.  A BPR-FM model's score is
-    <P[u], Q[i]> plus a term that is the same for every item of a user (``_user_offsets``); c0 is the batch-norm
-    model's share of that term, None for the other models."""
-    if isinstance(model, (BPRFM, BPRFMBN)):
-        return model.rank_tables()
-    return (*model._tables(), None)
-
-
-def _user_offsets(model, users, c0):
-    """b_u + bias_ (+ c0) per ranked user of a BPR-FM model: what ``forward()`` adds to every item of a user.  Call
-    only after ``model.check()``, so that an out-of-range user id raises there and never reaches this gather."""
-    off = model.biases.weight[users.long(), 0] + model.bias_
-    return off if c0 is None else off + c0
-
-
 def topk_candidates(model, users, cands, top_k):
     """users [N], cands [N, C] -> (pos [N,K] candidate positions, items [N,K], scores [N,K]) as device tensors.
-    ``model``: a dot-product model with ``_tables()`` (BPR, NCF(model='GMF')), a BPR-FM model (``BPRFM``, and
-    ``BPRFM(batch_norm=True)`` in evaluation mode), whose score is folded into one, or a ``NeuMF`` ('MLP' /
-    'NeuMF-end'), whose tower scores rank through ``daisy_neumf_topk_candidates``."""
-    neumf = isinstance(model, NeuMF)
-    bprfm = isinstance(model, (BPRFM, BPRFMBN))
-    dev = model._device() if neumf or bprfm else model._tables()[0].device
+    ``model``: a dot-product model (BPR, NCF(model='GMF')), a BPR-FM model (``BPRFM``, and ``BPRFM(batch_norm=True)`` in
+    evaluation mode), whose score is folded into one, or a ``NeuMF`` ('MLP' / 'NeuMF-end'), whose tower scores rank
+    through ``daisy_neumf_topk_candidates``; each ranks itself (``rank_candidates``)."""
+    dev = model._device()
     users = _i32(users, dev).reshape(-1)
     cands = _i32(cands, dev)
-    N, C = cands.shape
+    N, _ = cands.shape
     if users.shape[0] != N:
         raise ValueError("users and cands disagree on the number of groups")
-    h = model.handle()
-    pos = torch.empty((N, top_k), dtype=torch.int32, device=dev)
-    items = torch.empty((N, top_k), dtype=torch.int32, device=dev)
-    scores = torch.empty((N, top_k), dtype=torch.float32, device=dev)
-    out = (c_vp(pos.data_ptr()), c_vp(items.data_ptr()), c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev))
-    if neumf:
-        prm = model.params()
-        _lib.check(h.L.daisy_neumf_topk_candidates(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()),
-                                                   c_vp(cands.data_ptr()), N, C, int(top_k), *out))
-    else:
-        P, Q, c0 = _tables(model)
-        _lib.check(h.L.daisy_topk_candidates(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()),
-                                             c_vp(cands.data_ptr()), N, C, int(top_k), *out))
-    model.check()
-    if bprfm:
-        scores += _user_offsets(model, users, c0)[:, None]
-    return pos, items, scores
+    return model.rank_candidates(users, cands, top_k)
 
 
 def hr_ndcg(pos):
@@ -89,7 +49,7 @@ def metric_eval(model, test_loader, top_k, algo="bpr"):
     groups whose first candidate is the ground truth."""
     if algo not in ("bpr", "ncf"):
         raise ValueError("algo must be 'bpr' or 'ncf'")
-    if algo == "bpr" and isinstance(model, NeuMF):   # _bpr_topk calls model(user, item_i, item_j), which NCF does not take
+    if algo == "bpr" and not model.bpr_topk:
         raise ValueError("algo='bpr' needs a BPR model; rank an NCF model with algo='ncf'")
     groups = {}
     order = []
@@ -120,36 +80,9 @@ def topk_full(model, users, k, exclude=None):
     """Full-catalogue top-k for ``users``: (items [N,k] int32, scores [N,k]) device tensors, order (score desc, item asc).
     ``model``: BPR, NCF(model='GMF'), a BPR-FM model or a ``NeuMF``, as for ``topk_candidates``.
     ``exclude``: optional per-user lists of item ids to mask (training positives)."""
-    neumf = isinstance(model, NeuMF)
-    bprfm = isinstance(model, (BPRFM, BPRFMBN))
-    dev = model._device() if neumf or bprfm else model._tables()[0].device
+    dev = model._device()
     users = _i32(users, dev).reshape(-1)
-    N = users.shape[0]
-    h = model.handle()
-    items = torch.empty((N, k), dtype=torch.int32, device=dev)
-    scores = torch.empty((N, k), dtype=torch.float32, device=dev)
-    ptr_t = idx_t = None
-    if exclude is not None:
-        lens = np.fromiter((len(e) for e in exclude), dtype=np.int64, count=N)
-        ptr = np.zeros(N + 1, dtype=np.int64)
-        np.cumsum(lens, out=ptr[1:])
-        idx = np.concatenate([np.asarray(e, dtype=np.int32) for e in exclude]) if ptr[-1] else np.zeros(0, np.int32)
-        ptr_t = torch.from_numpy(ptr).to(dev)
-        idx_t = torch.from_numpy(idx).to(dev)
-    excl = (c_vp(ptr_t.data_ptr()) if ptr_t is not None else None,
-            c_vp(idx_t.data_ptr()) if idx_t is not None and idx_t.numel() else None)
-    out = (c_vp(items.data_ptr()), c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev))
-    if neumf:
-        prm = model.params()
-        _lib.check(h.L.daisy_neumf_topk_full(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()), N, int(k), *excl, *out))
-    else:
-        P, Q, c0 = _tables(model)
-        _lib.check(h.L.daisy_topk_full(h.ptr, c_vp(P.data_ptr()), c_vp(Q.data_ptr()), c_vp(users.data_ptr()), N, int(k),
-                                       *excl, *out))
-    model.check()
-    if bprfm:
-        scores += _user_offsets(model, users, c0)[:, None]
-    return items, scores
+    return model.rank_full(users, k, _lib.exclusion_csr(exclude, users.shape[0], dev))
 
 
 # ----------------------------------------------------------------------------------------------------------------

@@ -28,7 +28,7 @@ def _samples(user, item, label, device):
     return s.to(device=device, dtype=torch.int32).contiguous()
 
 
-class NCF(nn.Module):
+class NCF(_lib.HandleOwner, nn.Module):
     """``NCF(user_num, item_num, factor_num, num_layers, dropout, model)`` with ``model == 'GMF'``.
 
     Attributes as in the reference: ``embed_user_GMF``, ``embed_item_GMF`` (``nn.Embedding``, N(0, 0.01^2)) and
@@ -36,6 +36,9 @@ class NCF(nn.Module):
     ``forward(user, item) -> prediction`` (:105-125) runs ``daisy_gmf_forward``; training goes through
     ``GMFAdam.step`` (one fused pipeline), not autograd.
     """
+
+    _batch_grows = True
+    _cpu_error = "NCF tables are on the CPU: call model.cuda() first (no CPU fallback)"
 
     def __init__(self, user_num, item_num, factor_num, num_layers=3, dropout=0.0, model="GMF", GMF_model=None,
                  MLP_model=None, max_batch=256):
@@ -57,14 +60,16 @@ class NCF(nn.Module):
         for p in self.parameters():
             p.requires_grad_(False)
         self._max_batch = int(max_batch)
-        self._handle = None
+
+    def _weight(self):
+        return self.embed_user_GMF.weight
+
+    def _handle_dims(self):
+        return self.user_num, self.item_num, self.factor_num
 
     def _tensors(self):
-        P, Q = self.embed_user_GMF.weight, self.embed_item_GMF.weight
-        if not P.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("NCF tables are on the CPU: call model.cuda() first (no CPU fallback)")
-        return P, Q, self.predict_layer.weight, self.predict_layer.bias
+        self._device()
+        return self.embed_user_GMF.weight, self.embed_item_GMF.weight, self.predict_layer.weight, self.predict_layer.bias
 
     def _tables(self):
         """(P * w, Q): what the candidate top-K kernel ranks with -- <P[u] * w, Q[i]> = logit - b, and the bias does not
@@ -72,23 +77,8 @@ class NCF(nn.Module):
         P, Q, w, _ = self._tensors()
         return (P * w.reshape(1, -1)).contiguous(), Q
 
-    def handle(self, batch=None):
-        P = self._tensors()[0]
-        dev = P.device.index if P.device.index is not None else torch.cuda.current_device()
-        need = max(self._max_batch, int(batch or 0))
-        h = self._handle
-        if h is None or h.device_index != dev or h.max_batch < need:
-            if h is not None:
-                h.close()
-            self._max_batch = need
-            h = _lib.Handle(dev, self.user_num, self.item_num, self.factor_num, need, 0)
-            self._handle = h
-        return h
-
-    def check(self):
-        if self._handle is not None:
-            P = self._tensors()[0]
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, P.device)))
+    def rank_tables(self):
+        return (*self._tables(), None)
 
     def forward(self, user, item):
         P, Q, w, b = self._tensors()
@@ -100,17 +90,6 @@ class NCF(nn.Module):
                                          c_vp(b.data_ptr()), c_vp(s.data_ptr()), B, c_vp(pred.data_ptr()),
                                          _lib.stream_ptr(torch, P.device)))
         return pred.view(-1)
-
-    def __getstate__(self):
-        d = self.__dict__.copy()
-        d["_handle"] = None
-        return d
-
-    def _apply(self, fn, *a, **k):
-        if self._handle is not None:
-            self._handle.close()
-            self._handle = None
-        return super()._apply(fn, *a, **k)
 
 
 class GMFAdam:

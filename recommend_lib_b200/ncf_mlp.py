@@ -23,9 +23,12 @@ from .ncf import _samples
 c_vp = ctypes.c_void_p
 
 
-class NeuMF(nn.Module):
+class NeuMF(_lib.HandleOwner, nn.Module):
     """``NCF(user_num, item_num, factor_num, num_layers, dropout, model)`` with ``model in ('MLP', 'NeuMF-end')``;
     initialisation as ``_init_weight_`` (:68-84).  ``forward(user, item) -> prediction`` (:105-125)."""
+
+    _cpu_error = "NCF tables are on the CPU: call model.cuda() first (no CPU fallback)"
+    bpr_topk = False        # _bpr_topk calls model(user, item_i, item_j), which NCF does not take
 
     def __init__(self, user_num, item_num, factor_num, num_layers=3, dropout=0.0, model="NeuMF-end", GMF_model=None,
                  MLP_model=None):
@@ -61,9 +64,14 @@ class NeuMF(nn.Module):
                 m.bias.data.zero_()
         for p in self.parameters():
             p.requires_grad_(False)
-        self._handle = None
 
     # -- plumbing -----------------------------------------------------------------------------------------------------
+    def _weight(self):
+        return self.embed_user_MLP.weight
+
+    def _handle_dims(self):
+        return self.user_num, self.item_num, 4          # device, error flag, launch counter
+
     def linears(self):
         return [m for m in self.MLP_layers if isinstance(m, nn.Linear)]
 
@@ -77,26 +85,6 @@ class NeuMF(nn.Module):
             t[f"W{l}"], t[f"b{l}"] = m.weight, m.bias
         t["wp"], t["bp"] = self.predict_layer.weight, self.predict_layer.bias
         return t
-
-    def _device(self):
-        W = self.embed_user_MLP.weight
-        if not W.is_cuda:
-            _lib.require_cuda()
-            raise _lib.DaisyError("NCF tables are on the CPU: call model.cuda() first (no CPU fallback)")
-        return W.device
-
-    def handle(self):
-        dev = self._device()
-        idx = dev.index if dev.index is not None else torch.cuda.current_device()
-        if self._handle is None or self._handle.device_index != idx:
-            if self._handle is not None:
-                self._handle.close()
-            self._handle = _lib.Handle(idx, self.user_num, self.item_num, 4, 0)   # device, error flag, launch counter
-        return self._handle
-
-    def check(self):
-        if self._handle is not None:
-            _lib.check(self._handle.L.daisy_check(self._handle.ptr, _lib.stream_ptr(torch, self._device())))
 
     def params(self, lr=0.0, betas=(0.9, 0.999), eps=1e-8, moments=None):
         """The ``daisy_neumf_params`` block over this module's tensors (+ an optimizer's moment tensors)."""
@@ -133,16 +121,35 @@ class NeuMF(nn.Module):
                                            _lib.stream_ptr(torch, dev)))
         return pred.view(-1)
 
-    def __getstate__(self):
-        d = self.__dict__.copy()
-        d["_handle"] = None
-        return d
+    # -- ranking: the tower's scores through daisy_neumf_topk_candidates / daisy_neumf_topk_full ----------------------
+    def rank_candidates(self, users, cands, top_k):
+        h = self.handle()
+        N, C = cands.shape
+        dev = users.device
+        pos = torch.empty((N, top_k), dtype=torch.int32, device=dev)
+        items = torch.empty((N, top_k), dtype=torch.int32, device=dev)
+        scores = torch.empty((N, top_k), dtype=torch.float32, device=dev)
+        prm = self.params()
+        _lib.check(h.L.daisy_neumf_topk_candidates(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()), c_vp(cands.data_ptr()),
+                                                   N, C, int(top_k), c_vp(pos.data_ptr()), c_vp(items.data_ptr()),
+                                                   c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev)))
+        self.check()
+        return pos, items, scores
 
-    def _apply(self, fn, *a, **k):
-        if self._handle is not None:
-            self._handle.close()
-            self._handle = None
-        return super()._apply(fn, *a, **k)
+    def rank_full(self, users, k, excl):
+        h = self.handle()
+        N = users.shape[0]
+        dev = users.device
+        ptr, idx = excl
+        items = torch.empty((N, k), dtype=torch.int32, device=dev)
+        scores = torch.empty((N, k), dtype=torch.float32, device=dev)
+        prm = self.params()
+        _lib.check(h.L.daisy_neumf_topk_full(h.ptr, ctypes.byref(prm), c_vp(users.data_ptr()), N, int(k),
+                                             c_vp(ptr.data_ptr()) if ptr is not None else None,
+                                             c_vp(idx.data_ptr()) if idx is not None and idx.numel() else None,
+                                             c_vp(items.data_ptr()), c_vp(scores.data_ptr()), _lib.stream_ptr(torch, dev)))
+        self.check()
+        return items, scores
 
 
 class NeuMFAdam:

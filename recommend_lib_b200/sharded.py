@@ -513,22 +513,16 @@ class PeerShardedBPR:
         cands_global [N, C] (global item ids, ground truth first) -> candidate positions [N, K] in rank order.  The
         candidates' rows are fetched once from their owners; scores and the (score desc, position asc) order are those of
         ``daisy_topk_candidates`` on the unsharded tables."""
-        vp = self._lib.c_vp
         users = torch.as_tensor(np.asarray(users_local)).to(self.device, torch.int32).contiguous()
         cands = torch.as_tensor(np.asarray(cands_global)).to(self.device, torch.int64)
         N, C = cands.shape
-        pos = torch.empty((N, top_k), dtype=torch.int32, device=self.device)
         if N == 0:
-            return pos
+            return torch.empty((N, top_k), dtype=torch.int32, device=self.device)
         uniq, inv = torch.unique(cands.reshape(-1), return_inverse=True)
         cache = self.gather_item_rows(uniq)
         cidx = inv.reshape(N, C).to(torch.int32).contiguous()
         h = self._eval_handle(uniq.shape[0])
-        items = torch.empty((N, top_k), dtype=torch.int32, device=self.device)
-        scores = torch.empty((N, top_k), dtype=torch.float32, device=self.device)
-        self._lib.check(h.L.daisy_topk_candidates(h.ptr, vp(self._P_ptr), vp(cache.data_ptr()), vp(users.data_ptr()),
-                                                  vp(cidx.data_ptr()), N, C, int(top_k), vp(pos.data_ptr()),
-                                                  vp(items.data_ptr()), vp(scores.data_ptr()), self._s()))
+        pos, _, _ = self._lib.call_topk_candidates(h, self._P_ptr, cache.data_ptr(), users, cidx, top_k, self._s())
         self._lib.check(h.L.daisy_check(h.ptr, self._s()))
         return pos
 
@@ -555,7 +549,6 @@ class PeerShardedBPR:
         per-shard winners are merged -- scores are the exact fp32 scores and the order is (score desc, global item asc),
         so the result equals ``daisy_topk_full`` on the unsharded table.  Returns (items [N, k] int64 global ids,
         scores [N, k])."""
-        vp = self._lib.c_vp
         users = torch.as_tensor(np.asarray(users_local)).to(self.device, torch.int32).contiguous()
         N = users.shape[0]
         self.materialize()
@@ -576,20 +569,8 @@ class PeerShardedBPR:
                 buf[:rows].copy_(view)                     # the shard crosses NVLink once
                 q_local_ptr = buf.data_ptr()
             h = self._eval_handle(rows)
-            items = torch.empty((N, kk), dtype=torch.int32, device=self.device)
-            scores = torch.empty((N, kk), dtype=torch.float32, device=self.device)
-            ptr_t = idx_t = None
-            if exclude is not None:
-                ex = [np.asarray(e, dtype=np.int64) for e in exclude]
-                ex = [(e[(e >= i0) & (e < i1)] - i0).astype(np.int32) for e in ex]
-                ptr = np.zeros(N + 1, dtype=np.int64)
-                np.cumsum([len(e) for e in ex], out=ptr[1:])
-                idx = np.concatenate(ex) if ptr[-1] else np.zeros(0, np.int32)
-                ptr_t, idx_t = torch.from_numpy(ptr).to(self.device), torch.from_numpy(idx).to(self.device)
-            self._lib.check(h.L.daisy_topk_full(h.ptr, vp(self._P_ptr), vp(q_local_ptr), vp(users.data_ptr()), N, kk,
-                                                vp(ptr_t.data_ptr()) if ptr_t is not None else None,
-                                                vp(idx_t.data_ptr()) if idx_t is not None and idx_t.numel() else None,
-                                                vp(items.data_ptr()), vp(scores.data_ptr()), self._s()))
+            excl = self._lib.exclusion_csr(exclude, N, self.device, (i0, i1))
+            items, scores = self._lib.call_topk_full(h, self._P_ptr, q_local_ptr, users, kk, excl, self._s())
             self._lib.check(h.L.daisy_check(h.ptr, self._s()))
             all_items.append(items.to(torch.int64) + i0)
             all_scores.append(scores)

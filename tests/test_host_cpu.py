@@ -259,6 +259,24 @@ def test_neumf_module_is_a_drop_in_and_has_no_cpu_path():
             NeuMFAdam(m).step(z, z, torch.zeros(2))
 
 
+def test_ranking_refuses_cpu_tables():
+    """metrics.topk_candidates / topk_full hand the ranking to the model; every rankable model with its tables on the CPU
+    raises instead of ranking on the host."""
+    from recommend_lib_b200 import _lib, metrics
+    from recommend_lib_b200.bpr import BPR
+    from recommend_lib_b200.bprfm import BPRFM
+    from recommend_lib_b200.ncf import NCF
+    from recommend_lib_b200.ncf_mlp import NeuMF
+    U, I = 10, 12
+    models = [BPR(U, I, 8), NCF(U, I, 8), BPRFM(U + I, 8, user_num=U), BPRFM(U + I, 8, True, user_num=U).eval(),
+              NeuMF(U, I, 8)]
+    for m in models:
+        with pytest.raises(_lib.DaisyError, match="no CPU fallback"):
+            metrics.topk_candidates(m, [0, 1], [[1, 2, 3], [4, 5, 6]], 2)
+        with pytest.raises(_lib.DaisyError, match="no CPU fallback"):
+            metrics.topk_full(m, [0, 1], 2, exclude=[[1], []])
+
+
 def test_committed_bench_lines_carry_every_contract_key():
     """The JSON lines bench.py printed on a B200 at the end of round 2 (N = 1 at the default and at the driver's flags,
     N = 8 under torchrun) hold every key the bench contract names -- so a change to bench.py that drops one shows up here
